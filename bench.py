@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the Voice100 ASR hot path: log-mel + ConvVoiceEncoder + CTC head + greedy argmax.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Metric (BASELINE.json): ASR audio-seconds per second on `asr_en_base` (AudioToTextCTC(64,512,29,512)),
@@ -17,8 +17,8 @@ path over one batch.  Prints ONE JSON line on rank 0.
             lists every kernel class (depthwise and log-mel against the measured HBM copy bandwidth).
   cpu_baseline / --impl reference
             the CPU oracle (oracle/v100_oracle.py: the reference's arithmetic on torch CPU fp32, all host
-            threads) on a bounded sample of the same workload.  /root/reference itself is Python that
-            cannot travel to the GPU box; the oracle is pinned to it by tests/golden.
+            threads) on a bounded sample of the same workload.  The reference project is not part of this
+            repository; the oracle is pinned to its outputs by tests/golden.
 """
 import argparse
 import json
@@ -46,6 +46,33 @@ def load_peaks():
         return dict(hbm_gbs=p["hbm_gbs"], tf_burst=p["bf16_tflops"], tf_sustained=p["bf16_tflops_sustained"],
                     source="measured (MEASURED_PEAKS.json)")
     return dict(hbm_gbs=6650.0, tf_burst=1590.0, tf_sustained=1400.0, source="fallback (B200_PROFILING.md)")
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(directory, arrays):
+    """--dump-outputs: write what the timed path returned in its last step as <directory>/<name>.npy, floating point
+    as float32 and integers as float64 (exact), so that two builds can be compared output for output.  Every array is
+    batch-major; above DUMP_LIMIT_BYTES in all, the same seeded sample of utterances is kept from every array and
+    their batch indices are written as sample_rows.npy."""
+    import numpy as np
+    host = {}
+    for name, a in arrays.items():
+        a = a.detach().cpu().numpy() if hasattr(a, "detach") else np.asarray(a)
+        host[name] = a.astype(np.float32 if np.issubdtype(a.dtype, np.floating) else np.float64)
+    B = {a.shape[0] for a in host.values()}
+    assert len(B) == 1, {k: a.shape for k, a in host.items()}
+    B = B.pop()
+    total = sum(a.nbytes for a in host.values())
+    os.makedirs(directory, exist_ok=True)
+    if total > DUMP_LIMIT_BYTES:
+        keep = max(1, B * (DUMP_LIMIT_BYTES - 8 * B) // total)
+        rows = np.sort(np.random.default_rng(0).choice(B, keep, replace=False))
+        host = {k: a[rows] for k, a in host.items()}
+        np.save(os.path.join(directory, "sample_rows.npy"), rows.astype(np.float64))
+    for name, a in host.items():
+        np.save(os.path.join(directory, name + ".npy"), a)
 
 
 # --------------------------------------------------------------------------------------------------
@@ -176,14 +203,15 @@ def run_reference(args):
     step, threads = _cpu_pass_factory(batch)
     for _ in range(max(1, min(args.warmup, 2))):
         step()
-    steps = max(1, min(args.steps, 8))
+    steps = max(1, args.steps)
     t0 = time.perf_counter()
     for _ in range(steps):
-        step()
+        tokens = step()
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"tokens": tokens})
     value = steps * batch * CLIP_SECONDS / dt
-    sample = (f"each step = {batch} x {CLIP_SECONDS} s clips of the 256-clip workload on {threads} host threads "
-              f"(steps capped at 8 to bound the run)")
+    sample = f"each step = {batch} x {CLIP_SECONDS} s clips of the 256-clip workload on {threads} host threads"
     print(json.dumps({
         "impl": "reference", "metric": "asr_audio_seconds_per_second", "value": value, "unit": "audio-s/s",
         "n_gpus": args.gpus, "steps": steps, "warmup": args.warmup, "ms_per_step": 1e3 * dt / steps,
@@ -301,10 +329,15 @@ def run_tts(args):
     # The same two calls captured once into a CUDA graph (fixed shapes, device-resident inputs): an eager forward pays
     # one host round trip for the embedding's index check plus ~40 Python launches, which a slower host turns into
     # idle gaps between 20-200 us kernels (same kernels: 4.9 ms on one box, 5.7 ms on another).
+    outs = {}
+
     def both():
-        amodel(text_d)
-        vmodel.predict(at_d)
+        outs["align_pred"] = amodel(text_d)
+        outs["f0"], outs["logspc"], outs["codeap"] = vmodel.predict(at_d)
     ms, launch = _graph_leg(torch, dev, both, W, K, ms_eager)
+    if args.dump_outputs:
+        graphed = launch == "CUDA graph replay"
+        dump_outputs(args.dump_outputs, outs if graphed else dict(align_pred=pred, f0=f0, logspc=logspc, codeap=codeap))
     # end to end: host text in, host WORLD parameters out, host alignment loop in between
     Ke = max(2, min(K, 5))
     pin = lambda t: torch.empty(t.shape, dtype=t.dtype).pin_memory()
@@ -359,17 +392,23 @@ def run_tts_v2(args):
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
     for _ in range(K):
-        pred, _ = amodel(text_d, text_len)
+        pred, pred_len = amodel(text_d, text_len)
         f0, logspc, codeap = vmodel.predict(at_d, at_len)
     e1.record()
     torch.cuda.synchronize()
     ms_eager = e0.elapsed_time(e1) / K
     launches = (_lib.stats["launches"] - n0) // K
 
+    outs = {}
+
     def both():
-        amodel(text_d, text_len)
-        vmodel.predict(at_d, at_len)
+        outs["align_pred"], outs["align_pred_len"] = amodel(text_d, text_len)
+        outs["f0"], outs["logspc"], outs["codeap"] = vmodel.predict(at_d, at_len)
     ms, launch = _graph_leg(torch, dev, both, W, K, ms_eager)
+    if args.dump_outputs:
+        graphed = launch == "CUDA graph replay"
+        dump_outputs(args.dump_outputs, outs if graphed else dict(
+            align_pred=pred, align_pred_len=pred_len, f0=f0, logspc=logspc, codeap=codeap))
     Ke = max(2, min(K, 5))
     pin = lambda t: torch.empty(t.shape, dtype=t.dtype).pin_memory()
     pred_h, out_h, text_p = pin(pred), (pin(f0), pin(logspc), pin(codeap)), text.pin_memory()
@@ -434,6 +473,8 @@ def run_asr_v2(args):
         tokens, out_len = pipe(wavs[i & 1], lengths)
     e1.record()
     torch.cuda.synchronize()
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"tokens": tokens, "out_len": out_len})
     ms = e0.elapsed_time(e1) / K
     launches = (_lib.stats["launches"] - n0) // K
 
@@ -524,6 +565,9 @@ def main():
                          "then count valid samples only); the default is the metric's fixed 15 s clips")
     ap.add_argument("--vocab", type=int, default=MODEL["vocab_size"], help="44 = asr_ja_phone_base")
     ap.add_argument("--workload", default="asr", choices=["asr", "tts", "asr_v2", "tts_v2"], help="asr = the headline metric")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the arrays the timed path returned in its last step to DIR/<name>.npy "
+                         "(inputs are seeded: the same arguments give the same inputs on every run)")
     args = ap.parse_args()
     if args.impl == "reference":
         return run_reference(args)
@@ -626,6 +670,9 @@ def main():
         run.graph.replay()                      # launches_per_step kernels of libv100 per replay, nothing else
     e1.record()
     barrier()
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs if world == 1 else os.path.join(args.dump_outputs, f"rank{rank}"),
+                     {"tokens": run.tokens, "out_len": run.out_len})
     ms = e0.elapsed_time(e1)
     clocks = sampler.stop()
     ms_max = max_over_ranks(ms, dev)

@@ -193,6 +193,29 @@ def test_bench_work_model_matches_survey():
     assert 22e9 < big[0] < 25e9 and big[1] < 0.65 * big[0]           # ~23.5 GB per 256 x 15 s step, ~14 GB fused
 
 
+def test_bench_dump_outputs(tmp_path, monkeypatch):
+    """bench.py --dump-outputs: integers exactly as float64, floats as float32, and above the size limit the same
+    seeded utterances from every array, the same ones on every call."""
+    import sys
+    sys.path.insert(0, ROOT)
+    import bench
+    tok = torch.arange(40 * 7, dtype=torch.int64).view(40, 7)
+    logits = torch.randn(40, 7, 5, dtype=torch.float16)
+    bench.dump_outputs(str(tmp_path / "all"), {"tokens": tok, "logits": logits})
+    assert np.load(tmp_path / "all" / "tokens.npy").dtype == np.float64
+    assert np.array_equal(np.load(tmp_path / "all" / "tokens.npy"), tok.numpy())
+    assert np.array_equal(np.load(tmp_path / "all" / "logits.npy"), logits.float().numpy())
+    assert not (tmp_path / "all" / "sample_rows.npy").exists()
+    monkeypatch.setattr(bench, "DUMP_LIMIT_BYTES", 4096)
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), {"tokens": tok, "logits": logits})
+        assert sum(f.stat().st_size - 128 for f in (tmp_path / d).iterdir()) <= 4096   # minus the .npy headers
+    rows = np.load(tmp_path / "a" / "sample_rows.npy").astype(np.int64)
+    assert 0 < len(rows) < 40 and np.array_equal(rows, np.load(tmp_path / "b" / "sample_rows.npy"))
+    assert np.array_equal(np.load(tmp_path / "a" / "tokens.npy"), tok.numpy()[rows])
+    assert np.array_equal(np.load(tmp_path / "b" / "logits.npy"), logits.float().numpy()[rows])
+
+
 def test_load_checkpoint_roundtrip(tmp_path):
     """Lightning-style .ckpt (state_dict + hyper_parameters, plus training-only keys) -> drop-in module."""
     from collections import OrderedDict

@@ -4,7 +4,6 @@ against the oracle's mel pipeline."""
 import ctypes
 import os
 import subprocess
-import tempfile
 
 import numpy as np
 import pytest
@@ -48,19 +47,22 @@ extern "C" void rfft512_power_host(const float* frame, float* power) {
 
 
 @pytest.fixture(scope="module")
-def host_fft():
-    d = tempfile.mkdtemp()
+def host_lib(tmp_path_factory):
+    d = str(tmp_path_factory.mktemp("logmel_core"))
     src = os.path.join(d, "h.cpp")
     with open(src, "w") as f:
         f.write(HARNESS)
     so = os.path.join(d, "h.so")
     subprocess.check_call(["g++", "-O2", "-shared", "-fPIC", "-I", os.path.join(ROOT, "voice100_b200", "csrc"), "-o", so, src])
-    lib = ctypes.CDLL(so)
+    return ctypes.CDLL(so)
 
+
+@pytest.fixture(scope="module")
+def host_fft(host_lib):
     def run(frame):
         frame = np.ascontiguousarray(frame, np.float32)
         out = np.zeros(257, np.float32)
-        lib.rfft512_power_host(frame.ctypes.data_as(ctypes.c_void_p), out.ctypes.data_as(ctypes.c_void_p))
+        host_lib.rfft512_power_host(frame.ctypes.data_as(ctypes.c_void_p), out.ctypes.data_as(ctypes.c_void_p))
         return out
     return run
 
@@ -80,15 +82,12 @@ def test_rfft512_power_matches_numpy(host_fft):
     assert p.argmax() == 37 and abs(p[37] - 256.0 ** 2) < 1e-2 * 256.0 ** 2       # one bin, N/2 amplitude
 
 
-def test_fft16_matches_numpy(host_fft):
-    import glob
-    so = glob.glob(os.path.join(tempfile.gettempdir(), "*", "h.so"))
-    lib = ctypes.CDLL(sorted(so, key=os.path.getmtime)[-1])
+def test_fft16_matches_numpy(host_lib):
     rng = np.random.default_rng(1)
     for _ in range(5):
         v = (rng.standard_normal(16) + 1j * rng.standard_normal(16)).astype(np.complex64)
         buf = v.view(np.float32).copy()
-        lib.fft16_host(buf.ctypes.data_as(ctypes.c_void_p))
+        host_lib.fft16_host(buf.ctypes.data_as(ctypes.c_void_p))
         np.testing.assert_allclose(buf.view(np.complex64), np.fft.fft(v.astype(np.complex128)), atol=2e-6 * 16)
 
 
