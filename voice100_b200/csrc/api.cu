@@ -85,14 +85,14 @@ int make_tmap_3d(CUtensorMap* m, CUtensorMapDataType type, const void* base, int
   return encode(m, type, base, 3, dims, strides, box);
 }
 
-// NCW activations as a (T, C, B) tensor with an UNSWIZZLED box of [box_t steps x 1 channel x box_b utterances]: the
-// staged rows of one channel for several utterances in one TMA instruction, zero-filled outside [0, T) and [0, B).
+// NCW activations as a (T, C, B) tensor with a box of [box_t steps x 1 channel x box_b utterances]: the rows of one
+// channel for several utterances in one TMA instruction, zero-filled outside [0, T) and [0, B).
 int make_tmap_rows(CUtensorMap* m, CUtensorMapDataType type, const void* base, int64_t T, int64_t C, int64_t B,
-                   int64_t pitch_bytes, int box_t, int box_b) {
+                   int64_t pitch_bytes, int box_t, int box_b, CUtensorMapSwizzle swizzle) {
   const cuuint64_t dims[3] = {cuuint64_t(T), cuuint64_t(C), cuuint64_t(B)};
   const cuuint64_t strides[2] = {cuuint64_t(pitch_bytes), cuuint64_t(C) * cuuint64_t(pitch_bytes)};
   const cuuint32_t box[3] = {cuuint32_t(box_t), 1, cuuint32_t(box_b)};
-  return encode(m, type, base, 3, dims, strides, box, CU_TENSOR_MAP_SWIZZLE_NONE);
+  return encode(m, type, base, 3, dims, strides, box, swizzle);
 }
 
 }  // namespace v100

@@ -268,8 +268,18 @@ __device__ __forceinline__ void umma_bf16_cg2(uint32_t tmem_d, uint64_t desc_a, 
       ::"r"(tmem_d), "l"(desc_a), "l"(desc_b), "r"(idesc), "r"(accumulate)
       : "memory");
 }
-// Same with the A operand resident in TMEM ("TS" form): lane = row of this CTA's half of A, 16-bit elements packed
-// two per 32-bit column along K (one K = 16 step is 8 columns); only B comes from shared memory.
+// D[tmem] (+)= A[tmem] * B[smem desc] on one CTA ("TS" form): lane = row of A, 16-bit elements packed two per 32-bit
+// column along K (one K = 16 step is 8 columns); only B comes from shared memory.
+__device__ __forceinline__ void umma_ts(uint32_t tmem_d, uint32_t tmem_a, uint64_t desc_b, uint32_t idesc,
+                                        uint32_t accumulate) {
+  asm volatile(
+      "{\n\t.reg .pred p;\n\t"
+      "setp.ne.b32 p, %4, 0;\n\t"
+      "tcgen05.mma.cta_group::1.kind::f16 [%0], [%1], %2, %3, p;\n\t}"
+      ::"r"(tmem_d), "r"(tmem_a), "l"(desc_b), "r"(idesc), "r"(accumulate)
+      : "memory");
+}
+// The same pair form (cta_group::2): lane = row of this CTA's half of A.
 __device__ __forceinline__ void umma_ts_cg2(uint32_t tmem_d, uint32_t tmem_a, uint64_t desc_b, uint32_t idesc,
                                             uint32_t accumulate) {
   asm volatile(

@@ -49,7 +49,7 @@ int make_tmap_3d(CUtensorMap* m, CUtensorMapDataType type, const void* base, int
                  int64_t stride2_bytes, int box0, int box1);
 
 int make_tmap_rows(CUtensorMap* m, CUtensorMapDataType type, const void* base, int64_t T, int64_t C, int64_t B,
-                   int64_t pitch_bytes, int box_t, int box_b);
+                   int64_t pitch_bytes, int box_t, int box_b, CUtensorMapSwizzle swizzle = CU_TENSOR_MAP_SWIZZLE_NONE);
 
 int conv1x1(const void* x, int64_t x_pitch, const void* W, const float* scale, const float* shift, const void* res,
             void* y, int64_t y_pitch, int B, int C_in, int C_out, int T, int act, int dtype, cudaStream_t stream);
