@@ -142,12 +142,14 @@ def test_convtranspose_matches_torch(B, C_in, C_out, T, dtype):
 
 
 # ------------------------------------------------------------------------------------------------
-# depthwise conv (mma.sync Toeplitz kernel and the CUDA-core kernel)
+# depthwise conv (dw_tc_kernel, dw_bulk_kernel, the stride-2 kernels and the CUDA-core dw_simt_kernel)
 # ------------------------------------------------------------------------------------------------
 @pytest.mark.parametrize("k", [5, 7, 11, 17, 19, 27, 29, 33, 35, 51, 59, 65, 67, 75, 83])
 @pytest.mark.parametrize("T", [751, 96])
 @pytest.mark.parametrize("dtype", DTYPES)
 def test_dwconv_mma_matches_torch(k, T, dtype):
+    """Stride 1 through the default dispatch -- at T = 751 dw_bulk_kernel for k <= 33 and dw_tc_kernel from k = 35 up, at
+    T = 96 dw_tc_kernel for every k -- and through the CUDA-core dw_simt_kernel."""
     B, C = 2, 64
     x = rnd(B, C, T, seed=k).abs()
     w = rnd(C, k, seed=k + 1, scale=1.0 / math.sqrt(k)).to(dtype)
@@ -159,20 +161,23 @@ def test_dwconv_mma_matches_torch(k, T, dtype):
         y = K.dwconv(xn, w, scale, shift, k, 1, K.ACT_RELU6, simt=simt)
         torch.cuda.synchronize()
         assert y.T == T
-        assert rel_err(y.valid().float(), ref) < OUT_TOL[dtype], ("simt" if simt else "mma", rel_err(y.valid().float(), ref))
+        assert rel_err(y.valid().float(), ref) < OUT_TOL[dtype], ("simt" if simt else "default", rel_err(y.valid().float(), ref))
 
 
 @pytest.mark.parametrize("dtype", DTYPES)
 def test_dwconv_bulk_staging_edges(dtype):
-    """dw_bulk_kernel (filters of up to 59 taps): the row is staged by ONE cp.async.bulk + mbarrier per row.  Covered here:
-    every clip-length residue mod 8 (the bulk copy moves whole 16-byte groups, the last T & 7 samples come by plain loads
-    one row ahead), clips shorter than one group (no copy at all), rows of several 1024-output chunks with a partial last
-    one, batches that are not a multiple of the 8 rows a warp walks (both buffers and both barrier phases reused), garbage
-    in the pitch padding, and 300 repeats that must be bit-identical (the mbarrier protocol is not visible to racecheck)."""
+    """Row staging edges of the stride-1 kernels.  dw_bulk_kernel (k <= 33 on rows of 512 steps or more, C % 8 == 0) stages
+    each row by ONE cp.async.bulk + mbarrier; it takes (9, 24, 3001, 27), (17, 8, 1029, 11) and (5, 8, 756, 19): clip-length
+    residues mod 8 (the bulk copy moves whole 16-byte groups, the last T & 7 samples come by plain loads one row ahead),
+    rows of several 1024-output chunks with a partial last one, batches that are not a multiple of the 8 rows a warp walks
+    (both buffers and both barrier phases reused).  Every other shape here (k >= 35, or rows shorter than 512 steps)
+    takes dw_tc_kernel, whose zero-filled TMA boxes supply the halos and the clip tail.  Also: garbage in the pitch
+    padding, and 300 repeats (dw_tc_kernel, k = 59) that must be bit-identical (the mbarrier protocol is not visible to
+    racecheck)."""
     shapes = [(3, 16, 1027, 35), (11, 8, 2049, 59), (2, 8, 5, 19), (2, 8, 1, 5), (9, 24, 3001, 27), (2, 16, 1024, 51),
               (17, 8, 1029, 11), (2, 16, 1030, 51), (2, 8, 9, 59), (5, 8, 756, 19), (3, 8, 748, 43),
-              # short rows -> dw_rows_kernel (one TMA tensor load per channel and eight utterances): one and two boxes,
-              # fragments straddling the boxes, a batch that is not a multiple of eight, the longest filters
+              # short rows -> dw_tc_kernel (TMA boxes of 64 steps x up to 128 utterances): one to three 128-step tiles,
+              # a batch that is not a multiple of 16 (the MMA's N rounding), the longest filters
               (256, 16, 100, 29), (11, 8, 292, 65), (9, 8, 292, 33), (3, 8, 383, 83), (13, 8, 250, 5), (2, 8, 129, 11)]
     for B, C, T, k in shapes:
         x = rnd(B, C, T, seed=T + k)
@@ -200,7 +205,7 @@ def test_dwconv_bulk_staging_edges(dtype):
 
 @pytest.mark.parametrize("dtype", DTYPES)
 def test_dwconv_long_rows_and_stride2(dtype):
-    B, C, T, k = 2, 16, 3001, 83                       # 60 s clip: three 1024-output chunks per row
+    B, C, T, k = 2, 16, 3001, 83                       # 60 s clip: 24 dw_tc_kernel tiles of 128 steps per row
     x = rnd(B, C, T, seed=9)
     w = rnd(C, k, seed=10, scale=0.1).to(dtype)
     shift = torch.zeros(C, device=DEV)
