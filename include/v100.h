@@ -300,6 +300,54 @@ int64_t v100_lstm_workspace_bytes(int B, int H);
 int v100_lstm_layer(const void* gx, const void* w_hh, const int32_t* lengths, void* y, void* workspace,
                     int B, int Bp, int T, int H, int dtype, void* stream);
 
+/* ------------------------------------------------------------------------------------------------
+ * TTS text alignment
+ * ------------------------------------------------------------------------------------------------ */
+
+/* per-utterance status codes of v100_tts_align; the reference raises where noted */
+#define V100_ALIGN_OK       0
+#define V100_ALIGN_INDEX    1   /* rule 1: a frame index outside [-total, total)          (IndexError)    */
+#define V100_ALIGN_NEGATIVE 2   /* the total length is negative                            (RuntimeError)  */
+#define V100_ALIGN_NAN      3   /* the duration sum is NaN                                 (ValueError)    */
+#define V100_ALIGN_INF      4   /* the duration sum is +-inf                               (OverflowError) */
+#define V100_ALIGN_TOO_LONG 5   /* total >= 2^31 frames: frame indices are int32                           */
+#define V100_ALIGN_CAPACITY 6   /* total > T_cap: the first T_cap frames are written, the rest dropped      */
+
+/*
+ * Per-token (gap, duration) pairs -> aligned text, the int64 [B][T_cap] frame ids v100_embedding_ncw16 consumes.
+ * Replaces TextToAlignTextModel.align (voice100/models/tts.py:89-110, rule = 1) and TextToAlignText.align
+ * (voice100/models/_align_v2.py:54-82, rule = 2), each applied to one utterance at a time on the host, with the same
+ * results bit for bit:
+ *   rule 1: t = head + running sum of the entries in token order (float64); token i covers frames
+ *           [rint(t + gap_i), rint(t + gap_i + dur_i)), or [s, max(0, s + 1)) when the two are equal; later tokens
+ *           overwrite earlier ones; a frame j < 0 wraps to total + j; j outside [-total, total) is V100_ALIGN_INDEX.
+ *           total = head + int(sum) + tail.
+ *   rule 2: the first gap is skipped; s_i = max(trunc(t), e_{i-1}), e_i = max(trunc(t + dur_i), s_i + 1) (e_{-1} = 0);
+ *           frames at or past total are dropped.  total = head + int(sum - gap_0) + tail, the subtraction in fp32.
+ * The running position is summed by one thread per utterance, strictly in token order, as the reference's Python float
+ * is.  `sum` is the float32 rounding of the sequential float64 sum (the reference's CPU torch.sum may round differently
+ * when the sum lies within a few float32 ulps of an integer).
+ *   durations  fp32, element (b, i, c) at durations[b*stride_b + i*stride_l + c*stride_c], c = 0 gap, 1 duration;
+ *              this reads the align heads in place: the v1 NCW head [B][2][pitch] is (2*pitch, 1, pitch), the v2 dense
+ *              head over a time-major tensor ([1][2][pitch >= T*Bp], column t*Bp + b) is (1, Bp, pitch)
+ *   log1p_input  != 0: every value x is first replaced by expf(x) - 1, the exp(pred) - 1 the reference applies to the
+ *              head output (TextToAlignText.predict, _align_v2.py:45-48)
+ *   durations_out  optional fp32 [B][L][2]: the durations after that step, for all L tokens
+ *   text       int64 [B][L], row stride text_stride;  text_len  optional int32 [B] (NULL = L; clamped to [0, L])
+ *   aligntext  int64 [B][T_cap] or NULL (a plan-only call: lengths and status only, no capacity check); every element
+ *              of [0, T_cap) is written: frames of failed utterances and frames past the length are 0
+ *   aligntext_len  int32 [B]: the total length (also for V100_ALIGN_INDEX and V100_ALIGN_CAPACITY), 0 where undefined
+ *   status     int32 [B]: V100_ALIGN_*
+ *   filled_len optional int32 [B]: frames written = min(total, T_cap), 0 for a failed utterance (the LSTM lengths of
+ *              the v2 audio model);  frame_len  optional int32 [B]: 2*filled_len - 1 (0 if filled_len is 0), the WORLD
+ *              frames the audio models' stride-2 decoders produce from it
+ * L <= 4096 (V100_E_UNSUPPORTED above).  One CTA per utterance; no host synchronisation, CUDA-graph capturable.
+ */
+int v100_tts_align(const float* durations, int64_t stride_b, int64_t stride_l, int64_t stride_c, int log1p_input,
+                   float* durations_out, const int64_t* text, int64_t text_stride, const int32_t* text_len, int B,
+                   int L, int rule, int head, int tail, int64_t* aligntext, int T_cap, int32_t* aligntext_len,
+                   int32_t* status, int32_t* filled_len, int32_t* frame_len, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -11,11 +11,13 @@ every forward does, and fails loudly otherwise.
 from ._lib import V100Error, LIB_PATH  # noqa: F401
 from .data_modules import MelSpectrogramAudioTransform, BLANK_AUDIO, LOG_OFFSET, MELSPEC_DIM  # noqa: F401
 from .asr import AudioToTextCTC, ConvVoiceEncoder, LinearCharDecoder, AsrPipeline  # noqa: F401
-from .tts import TextToAlignTextModel, AlignTextToAudioModel, VoiceDecoder, WORLDNorm, align_batch  # noqa: F401
+from .tts import (TextToAlignTextModel, AlignTextToAudioModel, VoiceDecoder, WORLDNorm, align_batch,  # noqa: F401
+                  TtsPipeline)
 from .text import BasicTokenizer, CharTokenizer  # noqa: F401
 from .checkpoint import load_checkpoint  # noqa: F401
 from .align import ctc_best_path_batch  # noqa: F401
+from .kernels import align_frames  # noqa: F401
 from .audio import maskaudio  # noqa: F401
 from .v2 import (AudioToAlignText, TextToAlignText, AlignTextToAudio, AsrV2Pipeline,  # noqa: F401
-                 ConvLayerBlock, ConvTransposeLayerBlock, get_conv_layers, align_batch_v2)
+                 ConvLayerBlock, ConvTransposeLayerBlock, get_conv_layers, align_batch_v2, TtsV2Pipeline)
 from .vocoder import AlignTextToAudioPredict, create_mc2sp_matrix  # noqa: F401

@@ -40,6 +40,7 @@ SIGNATURES = {
     "v100_ncw_to_tm": [_p, _l, _p, _i, _i, _i, _i, _p],
     "v100_tm_to_ncw": [_p, _p, _l, _i, _i, _i, _i, _p],
     "v100_lstm_layer": [_p, _p, _p, _p, _p, _i, _i, _i, _i, _i, _p],
+    "v100_tts_align": [_p, _l, _l, _l, _i, _p, _p, _l, _p, _i, _i, _i, _i, _i, _p, _i, _p, _p, _p, _p, _p],
 }
 
 ABI_VERSION = 8

@@ -12,7 +12,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libv100.so")
-SOURCES = ["api.cu", "conv_gemm.cu", "fused_block.cu", "dwconv.cu", "logmel.cu", "misc.cu", "seq.cu", "lstm.cu"]
+SOURCES = ["api.cu", "conv_gemm.cu", "fused_block.cu", "dwconv.cu", "logmel.cu", "misc.cu", "seq.cu", "lstm.cu", "tts_align.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "--compiler-options", "-fPIC", "-shared"]
 

@@ -243,4 +243,13 @@ int v100_lstm_layer(const void* gx, const void* w_hh, const int32_t* lengths, vo
   return lstm_layer(gx, w_hh, lengths, y, workspace, B, Bp, T, H, dtype, STREAM(stream));
 }
 
+int v100_tts_align(const float* durations, int64_t stride_b, int64_t stride_l, int64_t stride_c, int log1p_input,
+                   float* durations_out, const int64_t* text, int64_t text_stride, const int32_t* text_len, int B,
+                   int L, int rule, int head, int tail, int64_t* aligntext, int T_cap, int32_t* aligntext_len,
+                   int32_t* status, int32_t* filled_len, int32_t* frame_len, void* stream) {
+  return tts_align(durations, stride_b, stride_l, stride_c, log1p_input, durations_out, text, text_stride, text_len, B,
+                   L, rule, head, tail, aligntext, T_cap, aligntext_len, status, filled_len, frame_len,
+                   STREAM(stream));
+}
+
 }  // extern "C"

@@ -105,4 +105,10 @@ size_t lstm_workspace_bytes(int B, int H);
 int lstm_layer(const void* gx, const void* w_hh, const int32_t* lengths, void* y, void* workspace, int B, int Bp,
                int T, int H, int dtype, cudaStream_t stream);
 
+// TTS text alignment (tts_align.cu)
+int tts_align(const float* durations, int64_t stride_b, int64_t stride_l, int64_t stride_c, int log1p_input,
+              float* durations_out, const int64_t* text, int64_t text_stride, const int32_t* text_len, int B, int L,
+              int rule, int head, int tail, int64_t* aligntext, int T_cap, int32_t* aligntext_len, int32_t* status,
+              int32_t* filled_len, int32_t* frame_len, cudaStream_t stream);
+
 }  // namespace v100

@@ -394,6 +394,103 @@ def tm_to_ncw(x: Tm) -> Ncw:
     return y
 
 
+# ---- TTS text alignment (v100_tts_align) ----
+
+ALIGN_OK, ALIGN_INDEX, ALIGN_NEGATIVE, ALIGN_NAN, ALIGN_INF, ALIGN_TOO_LONG, ALIGN_CAPACITY = range(7)   # V100_ALIGN_*
+ALIGN_FAILED = (ALIGN_INDEX, ALIGN_NEGATIVE, ALIGN_NAN, ALIGN_INF, ALIGN_TOO_LONG)
+
+
+def tts_align(text: torch.Tensor, align: torch.Tensor, text_len, rule: int, head: int, tail: int, T_cap,
+              log1p: bool, durations_out: torch.Tensor = None):
+    """One v100_tts_align call.  text int64 [B, L], align fp32 [B, L, 2] with any strides (a strided view of a head
+    output is read in place), text_len int32 [B] on the device or None.  T_cap None is a plan-only call.
+    -> (aligntext int64 [B, T_cap] or None, int32 [4, B] = aligntext_len, status, filled_len, frame_len)."""
+    if text.dtype != torch.int64 or not text.is_cuda or text.dim() != 2:
+        raise _lib.V100Error("tts_align: text must be a CUDA int64 [B, L] tensor")
+    if text.stride(1) != 1:
+        text = text.contiguous()                          # rows may be strided, tokens within a row may not
+    if align.dtype != torch.float32 or not align.is_cuda or align.dim() != 3 or align.shape[2] != 2:
+        raise _lib.V100Error("tts_align: align must be a CUDA fp32 [B, L, 2] tensor")
+    B, L = text.shape
+    if tuple(align.shape[:2]) != (B, L):
+        raise _lib.V100Error(f"tts_align: align {tuple(align.shape)} does not match text {tuple(text.shape)}")
+    if text_len is not None:
+        _cuda(text_len, torch.int32)
+    if durations_out is not None:
+        _cuda(durations_out, torch.float32)
+        if tuple(durations_out.shape) != (B, L, 2):
+            raise _lib.V100Error(f"tts_align: durations_out must be [{B}, {L}, 2]")
+    _same_device(text, align, text_len, durations_out)
+    dev = text.device
+    at = None if T_cap is None else torch.empty((B, T_cap), device=dev, dtype=torch.int64)
+    out = torch.empty((4, B), device=dev, dtype=torch.int32)
+    _call(text, "v100_tts_align", align.data_ptr(), align.stride(0), align.stride(1), align.stride(2),
+          1 if log1p else 0, _ptr(durations_out), text.data_ptr(), text.stride(0), _ptr(text_len), B, L, rule, head,
+          tail, _ptr(at), 0 if T_cap is None else T_cap, out[0].data_ptr(), out[1].data_ptr(), out[2].data_ptr(),
+          out[3].data_ptr())
+    return at, out
+
+
+def _raise_align_status(code: int, b: int):
+    """The exception the host loop raises for the utterance the kernel flagged."""
+    where = f"utterance {b}"
+    if code == ALIGN_INDEX:
+        raise IndexError(f"{where}: a frame index falls outside the aligned text (the reference loop raises here)")
+    if code == ALIGN_NEGATIVE:
+        raise RuntimeError(f"{where}: Trying to create tensor with negative dimension (the total length is negative)")
+    if code == ALIGN_NAN:
+        raise ValueError(f"{where}: cannot convert float NaN to integer (the duration sum is NaN)")
+    if code == ALIGN_INF:
+        raise OverflowError(f"{where}: cannot convert float infinity to integer (the duration sum is infinite)")
+    raise _lib.V100Error(f"{where}: the aligned text has 2^31 frames or more")
+
+
+def align_frames(text: torch.Tensor, align: torch.Tensor, text_len: torch.Tensor = None, rule: int = 1,
+                 head: int = 5, tail: int = 5, max_frames: int = None, log1p: bool = False,
+                 durations_out: torch.Tensor = None):
+    """Per-token (gap, duration) -> aligned text on the device: the batched, bit-exact form of
+    TextToAlignTextModel.align (rule=1, tts.py:89-110) and TextToAlignText.align (rule=2, _align_v2.py:54-82).
+    text int64 [B, L], align fp32 [B, L, 2] on the device (any strides), text_len [B] (None = all L tokens).
+    `log1p=True` applies exp(x) - 1 to `align` first (the head output is log(1 + duration)); `durations_out`, an
+    fp32 [B, L, 2] device tensor, then receives the durations.
+
+    Without `max_frames`: a plan call, one device-to-host copy of the lengths and status codes (8 bytes an utterance)
+    and an exact-size fill -> (aligntext int64 [B, max total], aligntext_len int32 [B]) on the device.  Where the host
+    loop fails, this raises the same exception class for the first such utterance (IndexError, RuntimeError,
+    ValueError, OverflowError).
+
+    With `max_frames`: one launch, no host synchronisation, nothing raised (CUDA-graph capturable) ->
+    (aligntext int64 [B, max_frames], aligntext_len int32 [B] clamped to max_frames, status int32 [B]).  status is
+    ALIGN_OK, one of ALIGN_FAILED (the row is all 0 and its length 0), or ALIGN_CAPACITY (the utterance was cut to
+    its first max_frames frames).
+
+    Rule 2 follows the reference loop where align_batch_v2 does not: frames at or past the total length are dropped
+    (the slice assignment of TextToAlignText.align), where align_batch_v2 raises IndexError."""
+    if rule not in (1, 2):
+        raise ValueError(f"rule must be 1 or 2, got {rule}")
+    dev = align.device
+    text = text.to(dev)
+    if text_len is not None:
+        text_len = text_len.to(device=dev, dtype=torch.int32).contiguous()
+    if max_frames is not None:
+        at, out = tts_align(text, align, text_len, rule, head, tail, int(max_frames), log1p, durations_out)
+        return at, out[2], out[1]
+    at, out = _align_exact(text, align, text_len, rule, head, tail, log1p, durations_out)
+    return at, out[0]
+
+
+def _align_exact(text, align, text_len, rule, head, tail, log1p, durations_out=None):
+    """Plan call, one device-to-host copy of (aligntext_len, status), then the fill at the batch's largest total.
+    Raises what the host loop raises for the first failing utterance.  -> tts_align's (aligntext, [4, B] lengths)."""
+    _, out = tts_align(text, align, text_len, rule, head, tail, None, log1p, durations_out)
+    plan = out[:2].cpu()                                  # the one host round trip
+    bad = (plan[1] != ALIGN_OK).nonzero()
+    if bad.numel():
+        b = int(bad[0, 0])
+        _raise_align_status(int(plan[1, b]), b)
+    return tts_align(text, align, text_len, rule, head, tail, int(plan[0].max()), log1p)
+
+
 def lstm_workspace(B: int, H: int, device) -> torch.Tensor:
     n = int(_lib.lib().v100_lstm_workspace_bytes(B, H))
     ws = torch.empty((n + 1024,), device=device, dtype=torch.uint8)

@@ -16,7 +16,7 @@ from .blocks import (InvertedResidualParams, PreparedCache, StorageDtypeMixin, r
                      run_inverted_residual)
 from .synth import ALIGN_KERNELS, VOICE_DECODER_POST_KERNELS, VOICE_DECODER_PRE_KERNELS
 
-__all__ = ["TextToAlignTextModel", "AlignTextToAudioModel", "VoiceDecoder", "WORLDNorm", "align_batch"]
+__all__ = ["TextToAlignTextModel", "AlignTextToAudioModel", "VoiceDecoder", "WORLDNorm", "align_batch", "TtsPipeline"]
 
 
 def _head(conv: nn.Conv1d, dtype):
@@ -37,14 +37,18 @@ class TextToAlignTextModel(StorageDtypeMixin, nn.Module):
             head=_head(self.layers[4], self.storage_dtype)))
         self.eval()
 
-    def forward(self, x: torch.Tensor) -> torch.Tensor:
-        """text int64 [B, L] -> fp32 [B, L, 2] = log(align + 1)."""
+    def _head_ncw(self, x: torch.Tensor) -> K.Ncw:
+        """text int64 [B, L] -> the head output as fp32 Ncw [B, 2, pitch] (rows: log(gap + 1), log(dur + 1))."""
         require_eval_cuda(self, x)
         w = self._prepared.get()
         h = K.embedding_ncw(x.contiguous(), w["table"])
         for blk in w["blocks"]:
             h = run_inverted_residual(h, blk)
-        return K.ncw_f32_to_ntc(K.conv1x1_f32(h, *w["head"]))
+        return K.conv1x1_f32(h, *w["head"])
+
+    def forward(self, x: torch.Tensor) -> torch.Tensor:
+        """text int64 [B, L] -> fp32 [B, L, 2] = log(align + 1)."""
+        return K.ncw_f32_to_ntc(self._head_ncw(x))
 
     def align(self, text: torch.Tensor, align: torch.Tensor, head: int = 5, tail: int = 5) -> torch.Tensor:
         """Host-side expansion of one utterance's tokens to 20 ms frames (tts.py:89-110): token i fills
@@ -208,3 +212,80 @@ class AlignTextToAudioModel(StorageDtypeMixin, nn.Module):
         mean, std = self._prepared.get()["norm"]
         _, f0, logspc, codeap = K.world_finalize(y, mean, std, True, self.logspc_size, self.codeap_size, 1)
         return f0, logspc, codeap
+
+
+class TtsPipeline:
+    """text -> WORLD parameters for TextToAlignTextModel + AlignTextToAudioModel, every stage a libv100 kernel and
+    the alignment on the device (v100_tts_align): align model -> exp(pred) - 1 and the frame expansion of
+    TextToAlignTextModel.align in one kernel -> audio model -> WORLD parameters.  Same results, bit for bit, as the
+    stepwise composition `align_model(text)` -> `torch.exp(pred) - 1` -> `align_batch` -> `audio_model.predict`.
+
+    `pipe(text, text_len=None, max_frames=None)` -> (f0 [B,T'], logspc [B,T',S], codeap [B,T',A], frame_len int32 [B],
+    status int32 [B]); frame_len = 2 * aligned length - 1 valid WORLD frames (0 for a failed utterance), status the
+    V100_ALIGN_* code (kernels.ALIGN_*).  Without `max_frames` the aligned text is sized to the batch's longest
+    utterance (one small host round trip) and an utterance the host loop fails on raises its exception; with
+    `max_frames` nothing waits on the host and nothing raises: utterances longer than max_frames frames are cut
+    (ALIGN_CAPACITY) and failed ones come back with frame_len 0.  `.graphed()` captures the whole path into one CUDA
+    graph.  The v1 models see the whole [B, L] text whatever `text_len` says (the reference's own behaviour):
+    text_len only limits which tokens are expanded into frames."""
+    rule = 1
+
+    def __init__(self, align_model, audio_model, head: int = 5, tail: int = 5):
+        self.align_model, self.audio_model, self.head, self.tail = align_model, audio_model, head, tail
+
+    def _durations(self, text: torch.Tensor, text_len):
+        """-> fp32 [B, L, 2] log(1 + (gap, duration)): a strided view of the head output, read in place."""
+        y = self.align_model._head_ncw(text)
+        return y.data.transpose(1, 2)[:, :text.shape[1]]
+
+    def _audio(self, aligntext: torch.Tensor, filled_len: torch.Tensor):
+        return self.audio_model.predict(aligntext)
+
+    @torch.no_grad()
+    def __call__(self, text: torch.Tensor, text_len: torch.Tensor = None, max_frames: int = None):
+        dev = next(self.align_model.parameters()).device
+        text = text.to(dev)
+        if text_len is not None:
+            text_len = text_len.to(device=dev, dtype=torch.int32)
+        pred = self._durations(text, text_len)
+        if max_frames is None:
+            at, lens = K._align_exact(text, pred, text_len, self.rule, self.head, self.tail, True)
+        else:
+            at, lens = K.tts_align(text, pred, text_len, self.rule, self.head, self.tail, int(max_frames), True)
+        f0, logspc, codeap = self._audio(at, lens[2])
+        return f0, logspc, codeap, lens[3], lens[1]
+
+    @torch.no_grad()
+    def graphed(self, batch: int, text_len_max: int, max_frames: int, device="cuda"):
+        """Capture text -> WORLD parameters for [batch, text_len_max] token ids and `max_frames` aligned frames into one
+        CUDA graph.  Returns `run(text, text_len=None) -> (f0, logspc, codeap, frame_len, status)`: `text` must be
+        [batch, text_len_max]; the outputs are static buffers overwritten by the next replay, and equal bit for bit
+        what `pipe(text, text_len, max_frames)` returns eagerly."""
+        dev = torch.device(device)
+        if dev.index is None:
+            dev = torch.device("cuda", torch.cuda.current_device())
+        with torch.cuda.device(dev):
+            text_s = torch.zeros((batch, text_len_max), dtype=torch.int64, device=dev)
+            len_s = torch.full((batch,), text_len_max, dtype=torch.int32, device=dev)
+            side = torch.cuda.Stream(dev)
+            side.wait_stream(torch.cuda.current_stream(dev))
+            with torch.cuda.stream(side):          # warm-up outside capture: prepared weights, function attributes
+                for _ in range(2):
+                    self(text_s, len_s, max_frames)
+            torch.cuda.current_stream(dev).wait_stream(side)
+            graph = torch.cuda.CUDAGraph()
+            with torch.cuda.graph(graph):
+                outs = self(text_s, len_s, max_frames)
+
+        def run(text: torch.Tensor, text_len: torch.Tensor = None):
+            if tuple(text.shape) != (batch, text_len_max):
+                raise V100Error(f"graphed TTS pipeline: text must be [{batch}, {text_len_max}], got {tuple(text.shape)}")
+            text_s.copy_(text, non_blocking=True)
+            if text_len is None:
+                len_s.fill_(text_len_max)
+            else:
+                len_s.copy_(text_len, non_blocking=True)
+            graph.replay()
+            return outs
+        run.graph, run.text, run.text_len, run.outputs = graph, text_s, len_s, outs
+        return run

@@ -23,10 +23,10 @@ from . import kernels as K
 from ._lib import V100Error
 from .asr import AsrPipeline
 from .blocks import PreparedCache, StorageDtypeMixin, require_eval_cuda
-from .tts import WORLDNorm
+from .tts import TtsPipeline, WORLDNorm
 
 __all__ = ["ConvLayerBlock", "ConvTransposeLayerBlock", "get_conv_layers", "AudioToAlignText", "TextToAlignText",
-           "AlignTextToAudio", "AsrV2Pipeline", "align_batch_v2"]
+           "AlignTextToAudio", "AsrV2Pipeline", "align_batch_v2", "TtsV2Pipeline"]
 
 
 class ConvLayerBlock(nn.Module):
@@ -271,13 +271,19 @@ class TextToAlignText(StorageDtypeMixin, nn.Module):
             lstm=_prepare_lstm(self.lstm, self.storage_dtype), head=_head(self.dense, self.storage_dtype)))
         self.eval()
 
-    def forward(self, text: torch.Tensor, text_len: torch.Tensor) -> Tuple[torch.Tensor, torch.Tensor]:
-        """text int64 [B, L], text_len [B] -> (fp32 [B, max_len, 2], lengths) (_align_v2.py:29-43)."""
+    def _head_tm(self, text: torch.Tensor, text_len: torch.Tensor):
+        """-> (fp32 head output over the time-major tensor, [1, 2, T*Bp] with column t*Bp + b, that tensor's
+        geometry); no host synchronisation."""
         require_eval_cuda(self, text)
         w = self._prepared.get()
         tm = K.ncw_to_tm(K.embedding_ncw(text.contiguous(), w["table"]))
         tm = _run_lstm(tm, w["lstm"], text_len)
-        y = _tm_head_to_tbc(K.conv1x1_f32(tm.as_ncw(), *w["head"]), tm)
+        return K.conv1x1_f32(tm.as_ncw(), *w["head"]), tm
+
+    def forward(self, text: torch.Tensor, text_len: torch.Tensor) -> Tuple[torch.Tensor, torch.Tensor]:
+        """text int64 [B, L], text_len [B] -> (fp32 [B, max_len, 2], lengths) (_align_v2.py:29-43)."""
+        y, tm = self._head_tm(text, text_len)
+        y = _tm_head_to_tbc(y, tm)
         t_max = min(int(text_len.max()), tm.T)
         return y[:t_max].transpose(0, 1).contiguous(), text_len.cpu()
 
@@ -377,10 +383,12 @@ class AlignTextToAudio(StorageDtypeMixin, nn.Module):
             norm=self.norm.packed()))
         self.eval()
 
-    def _decode(self, aligntext: torch.Tensor, aligntext_len: torch.Tensor) -> K.Ncw:
+    def _decode(self, aligntext: torch.Tensor, aligntext_len: torch.Tensor, t_max: int = None) -> K.Ncw:
+        """`t_max` (default: the longest length, read back from the device) = the steps the LSTM runs over."""
         require_eval_cuda(self, aligntext)
         w = self._prepared.get()
-        t_max = int(aligntext_len.max())                 # pad_packed_sequence trims to the longest utterance
+        if t_max is None:
+            t_max = int(aligntext_len.max())             # pad_packed_sequence trims to the longest utterance
         tm = K.ncw_to_tm(K.embedding_ncw(aligntext[:, :t_max].contiguous(), w["table"]))
         tm = _run_lstm(tm, w["lstm"], aligntext_len)
         x = self.decoder.run(K.tm_to_ncw(tm))
@@ -392,10 +400,35 @@ class AlignTextToAudio(StorageDtypeMixin, nn.Module):
         return K.world_finalize(self._decode(aligntext, aligntext_len), None, None, False, self.logspc_size,
                                 self.codeap_size, 2)
 
-    def predict(self, aligntext: torch.Tensor, aligntext_len: torch.Tensor):
+    def predict(self, aligntext: torch.Tensor, aligntext_len: torch.Tensor, t_max: int = None):
         """-> (f0 [B,T'], logspc [B,T',S], codeap [B,T',A]) un-normalised; f0 / codeap zeroed where their presence
-        logits are negative (_tts_v2.py:80-91) -- split, WORLDNorm.unnormalize and both `where`s in one kernel."""
-        y = self._decode(aligntext, aligntext_len)
+        logits are negative (_tts_v2.py:80-91) -- split, WORLDNorm.unnormalize and both `where`s in one kernel.
+        `t_max`: decode the first t_max frames without reading the lengths back (default max(aligntext_len))."""
+        y = self._decode(aligntext, aligntext_len, t_max)
         mean, std = self._prepared.get()["norm"]
         _, f0, logspc, _, codeap = K.world_finalize(y, mean, std, True, self.logspc_size, self.codeap_size, 2)
         return f0, logspc, codeap
+
+
+class TtsV2Pipeline(TtsPipeline):
+    """text -> WORLD parameters for TextToAlignText + AlignTextToAudio (or AlignTextToAudioPredict, the form the shipped
+    mel-cepstral tts_en_base.yaml needs): LSTM duration model -> exp(pred) - 1 and the frame expansion of
+    TextToAlignText.align in one kernel (v100_tts_align, reading the head output over the time-major tensor in place)
+    -> audio model -> WORLD parameters.  Same results, bit for bit, as `TextToAlignText.predict` -> `align_batch_v2` ->
+    `AlignTextToAudio.predict` wherever align_batch_v2 does not raise; where it raises because a token runs past the
+    total length, this follows `TextToAlignText.align` and drops those frames.  Same interface as TtsPipeline.
+
+    With `max_frames` the audio model's LSTM runs max_frames steps whatever the utterances' lengths (a captured graph
+    has fixed shapes).  A step is latency-bound and costs about 4 us, so keep the capacity close to the expected
+    longest utterance."""
+    rule = 2
+
+    def _durations(self, text: torch.Tensor, text_len):
+        if text_len is None:
+            text_len = torch.full((text.shape[0],), text.shape[1], dtype=torch.int32, device=text.device)
+        y, tm = self.align_model._head_tm(text, text_len)
+        return torch.as_strided(y.data, (tm.B, tm.T, 2), (1, tm.Bp, y.pitch))
+
+    def _audio(self, aligntext: torch.Tensor, filled_len: torch.Tensor):
+        m = self.audio_model
+        return (m.predict if isinstance(m, AlignTextToAudio) else m)(aligntext, filled_len, t_max=aligntext.shape[1])

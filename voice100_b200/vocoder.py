@@ -85,11 +85,13 @@ class AlignTextToAudioPredict(nn.Module):
         return dict(w=torch.cat(rows_w, 0).to(dtype).contiguous(), b=torch.cat(rows_b, 0).float().contiguous(),
                     bins=Wsp.shape[0], ident=(torch.zeros(n_out, device=dev), torch.ones(n_out, device=dev)))
 
-    def forward(self, aligntext: torch.Tensor, aligntext_len: torch.Tensor) -> Tuple[torch.Tensor, ...]:
+    def forward(self, aligntext: torch.Tensor, aligntext_len: torch.Tensor, t_max: int = None) -> Tuple[torch.Tensor, ...]:
+        """`t_max`: decode the first t_max frames without reading the lengths back (default max(aligntext_len))."""
         m = self.model
         require_eval_cuda(self, aligntext)
         w, mw = self._prepared.get(), m._prepared.get()
-        t_max = int(aligntext_len.max())
+        if t_max is None:
+            t_max = int(aligntext_len.max())
         tm = K.ncw_to_tm(K.embedding_ncw(aligntext[:, :t_max].contiguous(), mw["table"]))
         tm = _run_lstm(tm, mw["lstm"], aligntext_len)
         x = m.decoder.run(K.tm_to_ncw(tm))
