@@ -348,6 +348,74 @@ int v100_tts_align(const float* durations, int64_t stride_b, int64_t stride_l, i
                    int L, int rule, int head, int tail, int64_t* aligntext, int T_cap, int32_t* aligntext_len,
                    int32_t* status, int32_t* filled_len, int32_t* frame_len, void* stream);
 
+/* ------------------------------------------------------------------------------------------------
+ * WORLD waveform synthesis (fs = 16000, fft_size = 512, frame period 10 ms)
+ *
+ * Replaces WORLDVocoder.decode (voice100/vocoder.py:89-102): pyworld.decode_aperiodicity followed by
+ * pyworld.synthesize, i.e. WORLD's DecodeAperiodicity (codec.cpp) and Synthesis (synthesis.cpp), run on the host one
+ * utterance at a time.  The contract is the float64 restatement oracle/world.py; parity with pyworld itself has not
+ * been checked (DESIGN.md section 3.8 lists the details a restatement could have wrong).
+ * Inputs are fp32 device tensors read in place through strides (element strides):
+ *   f0      (b, t)    at f0[b*f0_sb + t*f0_st]                       Hz; < 32.25 (and negative) = unvoiced
+ *   logspc  (b, t, k) at logspc[b*sp_sb + t*sp_st + k*sp_sk], k < 257  natural log of the power spectrum (sp = exp)
+ *   codeap  (b, t)    at codeap[b*ap_sb + t*ap_st]                    coded aperiodicity, one band at 16 kHz
+ *   frame_len  optional int32 [B]: utterance b has min(max(frame_len[b], 0), T) frames (NULL = T)
+ * ------------------------------------------------------------------------------------------------ */
+
+/* per-utterance status codes of v100_world_timebase / v100_world_synthesize */
+#define V100_WORLD_OK        0
+#define V100_WORLD_SHORT     1   /* fewer than 2 frames (WORLD reads f0[-1] there)                           */
+#define V100_WORLD_NONFINITE 2   /* a NaN or inf in f0, logspc or codeap of the utterance's frames            */
+
+/*
+ * WORLD's randn() stream after its reseed (matlabfunctions.cpp randn / initializeSeed): xorshift128 with state
+ * (123456789, 362436069, 521288629, 88675123); value j sums (w >> 4) over 12 steps and is sum / 2^28 - 6, exact in
+ * float64.  out: float64 [n] on the device.  One thread runs the recurrence (about 12 n dependent steps); the table
+ * depends on n only, so build it once and keep it.
+ */
+int v100_world_noise(double* out, int64_t n, void* stream);
+
+/*
+ * Bytes of the workspace of v100_world_timebase / v100_world_synthesize for B utterances of at most y_len_max = 160 T
+ * samples; it does not depend on the WORLD parameters.  Layout, Yp = y_len_max rounded up to a multiple of 32:
+ *   int32 head[B][4]  (status, y_len, sample of the first pulse, number of pulses), padded to 256 bytes;
+ *   int32 info[B][Yp] -1 where no pulse sits at the sample, else (noise size << 1) | vuv, padded to 256 bytes;
+ *   double tau[B][Yp] the pulse's fractional time shift in s (defined at pulse samples only).
+ */
+int64_t v100_world_workspace_bytes(int B, int64_t y_len_max);
+
+/*
+ * The time base of Synthesis (GetTimeBase: GetTemporalParametersForTimeBase + interp1 + GetPulseLocationsForTimeBase)
+ * into the workspace, one CTA per utterance: f0 < 32.25 Hz is unvoiced, a knot at T is extrapolated
+ * (2 f[T-1] - f[T-2]), f0 and voicing are interpolated per sample with interp1's formula, vuv > 0.5 keeps f0 and
+ * anything else takes 500 Hz; the phase sum((2 pi) f0 / fs) is accumulated by one thread in sample order in float64
+ * and a pulse sits at sample i < y_len - 1 where |fmod(phi[i+1], 2 pi) - fmod(phi[i], 2 pi)| > pi.  No FMA
+ * contraction: the pulse samples and shifts equal oracle/world.py's bit for bit.
+ *   wav_len  int32 [B]: 160 frames (0 for a rejected utterance);  status  int32 [B]: V100_WORLD_*
+ */
+int v100_world_timebase(const float* f0, int64_t f0_sb, int64_t f0_st, const float* logspc, int64_t sp_sb,
+                        int64_t sp_st, int64_t sp_sk, const float* codeap, int64_t ap_sb, int64_t ap_st,
+                        const int32_t* frame_len, int B, int T, void* workspace, int32_t* wav_len, int32_t* status,
+                        void* stream);
+
+/*
+ * DecodeAperiodicity + Synthesis: v100_world_timebase, then one CTA per (1024-sample tile, utterance) computes every
+ * pulse response that reaches its tile (GetOneFrameSegment: spectral envelope and aperiodic ratio interpolated at the
+ * pulse, periodic part min-phase(log(S (1 - A) + eps) / 2) with the fractional delay and DC removal, aperiodic part
+ * min-phase(log(S A + eps) / 2) times the pulse's noise) in fp32 and adds them in pulse order.  Deterministic: the
+ * same inputs give the same bits in any batch.
+ *   noise      v100_world_noise output with noise_len >= 160 T values
+ *   workspace  v100_world_workspace_bytes(B, 160 T) bytes, 256-byte aligned
+ *   wav        fp32 [B][wav_pitch], wav_pitch >= 160 T: every sample of every row is written; samples at or past
+ *              wav_len[b], and whole rows of rejected utterances, are 0
+ *   wav_len, status as v100_world_timebase
+ */
+int v100_world_synthesize(const float* f0, int64_t f0_sb, int64_t f0_st, const float* logspc, int64_t sp_sb,
+                          int64_t sp_st, int64_t sp_sk, const float* codeap, int64_t ap_sb, int64_t ap_st,
+                          const int32_t* frame_len, int B, int T, const double* noise, int64_t noise_len,
+                          void* workspace, float* wav, int64_t wav_pitch, int32_t* wav_len, int32_t* status,
+                          void* stream);
+
 #ifdef __cplusplus
 }
 #endif

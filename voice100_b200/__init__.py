@@ -5,6 +5,7 @@ Drop-in module names follow the reference (kaiidams/voice100):
     voice100.models.asr.AudioToTextCTC                 -> voice100_b200.AudioToTextCTC
     voice100.models.tts.TextToAlignTextModel           -> voice100_b200.TextToAlignTextModel
     voice100.models.tts.AlignTextToAudioModel          -> voice100_b200.AlignTextToAudioModel
+    voice100.vocoder.WORLDVocoder (decode)             -> voice100_b200.WORLDVocoder
 All compute goes through libv100.so (include/v100.h); importing this package does not need a GPU, but
 every forward does, and fails loudly otherwise.
 """
@@ -20,4 +21,4 @@ from .kernels import align_frames  # noqa: F401
 from .audio import maskaudio  # noqa: F401
 from .v2 import (AudioToAlignText, TextToAlignText, AlignTextToAudio, AsrV2Pipeline,  # noqa: F401
                  ConvLayerBlock, ConvTransposeLayerBlock, get_conv_layers, align_batch_v2, TtsV2Pipeline)
-from .vocoder import AlignTextToAudioPredict, create_mc2sp_matrix  # noqa: F401
+from .vocoder import AlignTextToAudioPredict, create_mc2sp_matrix, WORLDVocoder  # noqa: F401

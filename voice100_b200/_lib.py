@@ -41,6 +41,10 @@ SIGNATURES = {
     "v100_tm_to_ncw": [_p, _p, _l, _i, _i, _i, _i, _p],
     "v100_lstm_layer": [_p, _p, _p, _p, _p, _i, _i, _i, _i, _i, _p],
     "v100_tts_align": [_p, _l, _l, _l, _i, _p, _p, _l, _p, _i, _i, _i, _i, _i, _p, _i, _p, _p, _p, _p, _p],
+    "v100_world_noise": [_p, _l, _p],
+    "v100_world_workspace_bytes": [_i, _l],   # returns int64 (restype set in lib())
+    "v100_world_timebase": [_p, _l, _l, _p, _l, _l, _l, _p, _l, _l, _p, _i, _i, _p, _p, _p, _p],
+    "v100_world_synthesize": [_p, _l, _l, _p, _l, _l, _l, _p, _l, _l, _p, _i, _i, _p, _l, _p, _p, _l, _p, _p, _p],
 }
 
 ABI_VERSION = 8
@@ -65,6 +69,7 @@ def lib():
             fn.restype = _i
         handle.v100_lstm_workspace_bytes.argtypes = [_i, _i]
         handle.v100_lstm_workspace_bytes.restype = _l
+        handle.v100_world_workspace_bytes.restype = _l
         handle.v100_last_error.argtypes = []
         handle.v100_last_error.restype = C.c_char_p
         if handle.v100_abi_version() != ABI_VERSION:
@@ -79,6 +84,8 @@ KERNELS_PER_CALL = {name: 1 for name in SIGNATURES}
 KERNELS_PER_CALL["v100_convtranspose1d_k5s2"] = 2
 KERNELS_PER_CALL["v100_conv1d"] = 2   # tap stacking + GEMM
 KERNELS_PER_CALL["v100_abi_version"] = 0
+KERNELS_PER_CALL["v100_world_synthesize"] = 2   # time base + synthesis
+KERNELS_PER_CALL["v100_world_workspace_bytes"] = 0
 
 stats = {"launches": 0}
 tracer = None  # optional object with before(name)/after(name), used by bench.py for per-kernel CUDA events

@@ -252,4 +252,25 @@ int v100_tts_align(const float* durations, int64_t stride_b, int64_t stride_l, i
                    STREAM(stream));
 }
 
+int v100_world_noise(double* out, int64_t n, void* stream) { return world_noise(out, n, STREAM(stream)); }
+
+int64_t v100_world_workspace_bytes(int B, int64_t y_len_max) { return world_workspace_bytes(B, y_len_max); }
+
+int v100_world_timebase(const float* f0, int64_t f0_sb, int64_t f0_st, const float* logspc, int64_t sp_sb,
+                        int64_t sp_st, int64_t sp_sk, const float* codeap, int64_t ap_sb, int64_t ap_st,
+                        const int32_t* frame_len, int B, int T, void* workspace, int32_t* wav_len, int32_t* status,
+                        void* stream) {
+  return world_timebase(f0, f0_sb, f0_st, logspc, sp_sb, sp_st, sp_sk, codeap, ap_sb, ap_st, frame_len, B, T,
+                        workspace, wav_len, status, STREAM(stream));
+}
+
+int v100_world_synthesize(const float* f0, int64_t f0_sb, int64_t f0_st, const float* logspc, int64_t sp_sb,
+                          int64_t sp_st, int64_t sp_sk, const float* codeap, int64_t ap_sb, int64_t ap_st,
+                          const int32_t* frame_len, int B, int T, const double* noise, int64_t noise_len,
+                          void* workspace, float* wav, int64_t wav_pitch, int32_t* wav_len, int32_t* status,
+                          void* stream) {
+  return world_synthesize(f0, f0_sb, f0_st, logspc, sp_sb, sp_st, sp_sk, codeap, ap_sb, ap_st, frame_len, B, T, noise,
+                          noise_len, workspace, wav, wav_pitch, wav_len, status, STREAM(stream));
+}
+
 }  // extern "C"

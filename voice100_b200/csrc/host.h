@@ -111,4 +111,15 @@ int tts_align(const float* durations, int64_t stride_b, int64_t stride_l, int64_
               int rule, int head, int tail, int64_t* aligntext, int T_cap, int32_t* aligntext_len, int32_t* status,
               int32_t* filled_len, int32_t* frame_len, cudaStream_t stream);
 
+// WORLD synthesis (world.cu)
+int64_t world_workspace_bytes(int B, int64_t y_len_max);
+int world_noise(double* out, int64_t n, cudaStream_t stream);
+int world_timebase(const float* f0, int64_t f0_sb, int64_t f0_st, const float* logspc, int64_t sp_sb, int64_t sp_st,
+                   int64_t sp_sk, const float* codeap, int64_t ap_sb, int64_t ap_st, const int32_t* frame_len, int B,
+                   int T, void* workspace, int32_t* wav_len, int32_t* status, cudaStream_t stream);
+int world_synthesize(const float* f0, int64_t f0_sb, int64_t f0_st, const float* logspc, int64_t sp_sb,
+                     int64_t sp_st, int64_t sp_sk, const float* codeap, int64_t ap_sb, int64_t ap_st,
+                     const int32_t* frame_len, int B, int T, const double* noise, int64_t noise_len, void* workspace,
+                     float* wav, int64_t wav_pitch, int32_t* wav_len, int32_t* status, cudaStream_t stream);
+
 }  // namespace v100

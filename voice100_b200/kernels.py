@@ -511,3 +511,112 @@ def lstm_layer(x: Tm, w_ih: torch.Tensor, bias: torch.Tensor, w_hh: torch.Tensor
     _call(x, "v100_lstm_layer", gx.data.data_ptr(), w_hh.data_ptr(), lengths.data_ptr(), y.data_ptr(),
               ws.data_ptr(), x.B, x.Bp, x.T, H, dt(x.data))
     return Tm(y, x.B, x.T, x.Bp)
+
+
+# ---------------------------------------------------------------------------------------------- WORLD synthesis
+
+WORLD_OK, WORLD_SHORT, WORLD_NONFINITE = 0, 1, 2      # V100_WORLD_*
+WORLD_FS, WORLD_FFT, WORLD_HOP, WORLD_BINS = 16000, 512, 160, 257
+_WORLD_NOISE_MIN = 1 << 20                            # values (65 s of audio) in the first table of a device
+_world_noise = {}                                     # device index -> float64 table (WORLD's randn stream)
+_world_noise_retired = []                             # replaced tables stay alive: captured graphs may still read them
+
+
+def world_noise(n: int, device) -> torch.Tensor:
+    """WORLD's randn() stream (v100_world_noise) as a float64 device tensor of at least n values, built once per
+    device and grown (to at least twice its size) when a longer one is needed.  Growing launches a kernel and allocates,
+    so it must happen outside CUDA-graph capture: a captured call that needs more than the table holds raises."""
+    dev = torch.device(device)
+    if dev.index is None:
+        dev = torch.device("cuda", torch.cuda.current_device())
+    tab = _world_noise.get(dev.index)
+    if tab is None or tab.numel() < n:
+        if torch.cuda.is_current_stream_capturing():
+            raise _lib.V100Error(f"the WORLD noise table holds {0 if tab is None else tab.numel()} values and {n} are "
+                                 "needed: run the call once before graph capture so that the table is built there")
+        m = max(int(n), _WORLD_NOISE_MIN, 2 * (0 if tab is None else tab.numel()))
+        new = torch.empty((m,), device=dev, dtype=torch.float64)
+        _call(new, "v100_world_noise", new.data_ptr(), m)
+        if tab is not None:
+            _world_noise_retired.append(tab)
+        _world_noise[dev.index] = tab = new
+    return tab
+
+
+def _world_inputs(f0, logspc, codeap, frame_len):
+    if f0.dim() != 2 or logspc.dim() != 3:
+        raise _lib.V100Error(f"WORLD synthesis: f0 must be [B, T] and logspc [B, T, {WORLD_BINS}]")
+    if codeap.dim() == 2:
+        codeap = codeap.unsqueeze(-1)
+    B, T = f0.shape
+    if logspc.shape[2] != WORLD_BINS:
+        raise _lib.V100Error(f"WORLD synthesis: logspc has {logspc.shape[2]} bins; the 16 kHz / 512-point vocoder "
+                             f"needs {WORLD_BINS} (25 mel-cepstra: decode them with AlignTextToAudioPredict)")
+    if codeap.dim() != 3 or codeap.shape[2] != 1:
+        raise _lib.V100Error(f"WORLD synthesis: codeap must be [B, T, 1] (one band at 16 kHz), got {tuple(codeap.shape)}")
+    if tuple(logspc.shape[:2]) != (B, T) or tuple(codeap.shape[:2]) != (B, T):
+        raise _lib.V100Error(f"WORLD synthesis: shapes f0 {tuple(f0.shape)}, logspc {tuple(logspc.shape)}, codeap "
+                             f"{tuple(codeap.shape)} do not agree")
+    for t in (f0, logspc, codeap):
+        if t.dtype != torch.float32 or not t.is_cuda:
+            raise _lib.V100Error("WORLD synthesis: f0, logspc and codeap must be fp32 CUDA tensors")
+    if frame_len is not None:
+        _cuda(frame_len, torch.int32)
+        if tuple(frame_len.shape) != (B,):
+            raise _lib.V100Error(f"WORLD synthesis: frame_len must be int32 [{B}]")
+    _same_device(f0, logspc, codeap, frame_len)
+    if B <= 0:
+        raise _lib.V100Error("WORLD synthesis: empty batch")
+    return B, T, codeap
+
+
+def _world_workspace(B: int, T: int, device) -> torch.Tensor:
+    n = int(_lib.lib().v100_world_workspace_bytes(B, WORLD_HOP * T))
+    ws = torch.empty((n + 256,), device=device, dtype=torch.uint8)
+    off = (-ws.data_ptr()) % 256
+    return ws[off:off + n]
+
+
+def _world_args(f0, logspc, codeap, frame_len):
+    return (f0.data_ptr(), f0.stride(0), f0.stride(1), logspc.data_ptr(), logspc.stride(0), logspc.stride(1),
+            logspc.stride(2), codeap.data_ptr(), codeap.stride(0), codeap.stride(1), _ptr(frame_len))
+
+
+def world_timebase(f0: torch.Tensor, logspc: torch.Tensor, codeap: torch.Tensor, frame_len: torch.Tensor = None):
+    """v100_world_timebase alone, decoded for inspection: -> (workspace views) dict with
+    head int32 [B, 4] (status, y_len, first pulse, pulse count), info int32 [B, 160 T] (-1, or noise size << 1 | vuv),
+    tau float64 [B, 160 T], wav_len int32 [B], status int32 [B]."""
+    B, T, codeap = _world_inputs(f0, logspc, codeap, frame_len)
+    Yp = (WORLD_HOP * T + 31) // 32 * 32
+    ws = _world_workspace(B, T, f0.device)
+    out = torch.empty((2, B), device=f0.device, dtype=torch.int32)
+    _call(f0, "v100_world_timebase", *_world_args(f0, logspc, codeap, frame_len), B, T, ws.data_ptr(),
+          out[0].data_ptr(), out[1].data_ptr())
+    a = lambda x: (x + 255) // 256 * 256
+    o1, o2 = a(B * 16), a(B * 16) + a(B * Yp * 4)
+    return dict(head=ws[:B * 16].view(torch.int32).view(B, 4), info=ws[o1:o1 + B * Yp * 4].view(torch.int32).view(B, Yp),
+                tau=ws[o2:o2 + B * Yp * 8].view(torch.float64).view(B, Yp), wav_len=out[0], status=out[1])
+
+
+def world_synthesize(f0: torch.Tensor, logspc: torch.Tensor, codeap: torch.Tensor, frame_len: torch.Tensor = None,
+                     max_samples: int = None):
+    """WORLD vocoder on the device (v100_world_synthesize): DecodeAperiodicity + Synthesis at 16 kHz, 512-point FFT,
+    10 ms frames, for a padded batch.  f0 fp32 [B, T] (Hz, 0 = unvoiced), logspc fp32 [B, T, 257], codeap fp32 [B, T, 1]
+    or [B, T], any strides (read in place); frame_len int32 [B] valid frames (None = T).
+    -> (wav fp32 [B, Y], wav_len int32 [B] = 160 frame_len, status int32 [B] = WORLD_*), Y = max_samples (>= 160 T,
+    default 160 T).  Samples from wav_len on are 0; a rejected utterance (WORLD_SHORT: fewer than two frames,
+    WORLD_NONFINITE: NaN / inf among its parameters) is all 0 with wav_len 0.  No host synchronisation; capturable once
+    the noise table of this device is large enough (see world_noise)."""
+    B, T, codeap = _world_inputs(f0, logspc, codeap, frame_len)
+    Y = WORLD_HOP * T if max_samples is None else int(max_samples)
+    if Y < WORLD_HOP * T or Y <= 0:
+        raise _lib.V100Error(f"world_synthesize: max_samples = {Y} must be positive and at least 160 T = "
+                             f"{WORLD_HOP * T}")
+    dev = f0.device
+    noise = world_noise(WORLD_HOP * T, dev)
+    ws = _world_workspace(B, T, dev)
+    wav = torch.empty((B, Y), device=dev, dtype=torch.float32)
+    out = torch.empty((2, B), device=dev, dtype=torch.int32)
+    _call(f0, "v100_world_synthesize", *_world_args(f0, logspc, codeap, frame_len), B, T, noise.data_ptr(),
+          noise.numel(), ws.data_ptr(), wav.data_ptr(), Y, out[0].data_ptr(), out[1].data_ptr())
+    return wav, out[0], out[1]

@@ -256,11 +256,28 @@ class TtsPipeline:
         return f0, logspc, codeap, lens[3], lens[1]
 
     @torch.no_grad()
-    def graphed(self, batch: int, text_len_max: int, max_frames: int, device="cuda"):
+    def waveform(self, text: torch.Tensor, text_len: torch.Tensor = None, max_frames: int = None):
+        """text -> 16 kHz PCM: the pipeline, then WORLD synthesis on the device (kernels.world_synthesize), in place of
+        the reference's WORLDVocoder.decode per utterance.  -> (wav fp32 [B, 160 T'], wav_len int32 [B] = 160
+        frame_len, status int32 [B] = kernels.WORLD_*).  `text_len` and `max_frames` as for `pipe(...)`: without
+        max_frames the exact-size path and its exceptions; with it no host synchronisation, and an utterance whose
+        alignment failed (frame_len 0) comes back as WORLD_SHORT with no samples.  Needs 257 log-spectrum bins (a
+        25-coefficient mel-cepstral model goes through AlignTextToAudioPredict)."""
+        f0, logspc, codeap, frame_len, _ = self(text, text_len, max_frames)
+        if logspc.shape[-1] != K.WORLD_BINS:
+            raise V100Error(f"TTS waveform: the audio model emits {logspc.shape[-1]} spectral coefficients; WORLD "
+                            f"synthesis needs {K.WORLD_BINS} log-spectrum bins (wrap a mel-cepstral AlignTextToAudio "
+                            "in AlignTextToAudioPredict)")
+        return K.world_synthesize(f0, logspc, codeap, frame_len)
+
+    @torch.no_grad()
+    def graphed(self, batch: int, text_len_max: int, max_frames: int, device="cuda", waveform: bool = False):
         """Capture text -> WORLD parameters for [batch, text_len_max] token ids and `max_frames` aligned frames into one
         CUDA graph.  Returns `run(text, text_len=None) -> (f0, logspc, codeap, frame_len, status)`: `text` must be
         [batch, text_len_max]; the outputs are static buffers overwritten by the next replay, and equal bit for bit
-        what `pipe(text, text_len, max_frames)` returns eagerly."""
+        what `pipe(text, text_len, max_frames)` returns eagerly.  With `waveform=True` the graph runs text -> PCM and
+        `run` returns what `pipe.waveform(text, text_len, max_frames)` returns: (wav, wav_len, status)."""
+        fn = self.waveform if waveform else self
         dev = torch.device(device)
         if dev.index is None:
             dev = torch.device("cuda", torch.cuda.current_device())
@@ -271,11 +288,11 @@ class TtsPipeline:
             side.wait_stream(torch.cuda.current_stream(dev))
             with torch.cuda.stream(side):          # warm-up outside capture: prepared weights, function attributes
                 for _ in range(2):
-                    self(text_s, len_s, max_frames)
+                    fn(text_s, len_s, max_frames)
             torch.cuda.current_stream(dev).wait_stream(side)
             graph = torch.cuda.CUDAGraph()
             with torch.cuda.graph(graph):
-                outs = self(text_s, len_s, max_frames)
+                outs = fn(text_s, len_s, max_frames)
 
         def run(text: torch.Tensor, text_len: torch.Tensor = None):
             if tuple(text.shape) != (batch, text_len_max):

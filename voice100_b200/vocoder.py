@@ -1,11 +1,12 @@
-"""Mel-cepstrum -> log-spectrum on the inference path (SURVEY.md section 8f #4).
+"""Mel-cepstrum -> log-spectrum on the inference path (SURVEY.md section 8f #4), and the WORLD vocoder.
 
 The reference's shipped TTS config trains AlignTextToAudio on 25 mel-cepstral coefficients (config/tts_en_base.yaml:29
 `vocoder: world_mcep`) and converts them back with a fixed matrix after `predict`
 (voice100/export_onnx.py:81-97 `AlignTextToAudioPredict`, voice100/vocoder.py:115-123 `create_mc2sp_matrix`).
 Un-normalisation and that matrix are both linear, so here they are folded into the projection layer: the head GEMM
 emits the 257 log-spectrum bins directly and the conversion costs nothing at run time.
-WORLD waveform synthesis itself (pyworld, a CPU C library) stays out of scope.
+WORLD waveform synthesis (the reference's WORLDVocoder.decode, pyworld on the host) runs on the device through
+`WORLDVocoder` (v100_world_synthesize); WORLD analysis (encode) is not on the inference path and stays out of scope.
 """
 from __future__ import annotations
 
@@ -99,3 +100,46 @@ class AlignTextToAudioPredict(nn.Module):
         _, f0, logspc, _, codeap = K.world_finalize(K.conv1x1_f32(x, w["w"], w["b"]), w["ident"][0], w["ident"][1],
                                                     True, w["bins"], m.codeap_size, 2)
         return f0, logspc, codeap
+
+
+class WORLDVocoder:
+    """WORLD synthesis on the device, in place of the reference's WORLDVocoder.decode (voice100/vocoder.py:89-102:
+    pyworld.decode_aperiodicity + pyworld.synthesize, one utterance on a CPU core).  Only the configuration every model
+    here emits is implemented: 16 kHz, 10 ms frames, 512-point FFT (257 log-spectrum bins, one coded-aperiodicity band).
+    The algorithm is the restatement in oracle/world.py; parity with pyworld itself is unverified (DESIGN.md 3.8).
+    Inputs are used as fp32, the precision the models produce them in."""
+
+    def __init__(self, sample_rate: int = 16000, frame_period: float = 10.0, n_fft: int = 512) -> None:
+        if (sample_rate, float(frame_period), n_fft) != (K.WORLD_FS, 10.0, K.WORLD_FFT):
+            raise V100Error(f"WORLDVocoder: only sample_rate=16000, frame_period=10.0, n_fft=512 is implemented "
+                            f"(got {sample_rate}, {frame_period}, {n_fft})")
+        self.sample_rate, self.frame_period, self.n_fft = sample_rate, float(frame_period), n_fft
+
+    def decode_batch(self, f0: torch.Tensor, logspc: torch.Tensor, codeap: torch.Tensor, frame_len: torch.Tensor = None,
+                     max_samples: int = None):
+        """Device tensors f0 [B, T], logspc [B, T, 257], codeap [B, T, 1] (fp32, any strides), frame_len int32 [B] or
+        None -> (wav fp32 [B, Y], wav_len int32 [B], status int32 [B]); see kernels.world_synthesize.  No host sync."""
+        if frame_len is not None:
+            frame_len = frame_len.to(device=f0.device, dtype=torch.int32).contiguous()
+        return K.world_synthesize(f0, logspc, codeap, frame_len, max_samples)
+
+    def decode(self, f0, logspc, codeap, device=None) -> np.ndarray:
+        """One utterance, like the reference: f0 [T], logspc [T, 257], codeap [T, 1] (numpy arrays or tensors)
+        -> float64 numpy waveform [160 T].  Runs on `device` (default: the tensors' CUDA device, else the current one).
+        Raises ValueError where WORLD has no defined behaviour (fewer than two frames, NaN or inf)."""
+        if device is None:
+            device = f0.device if isinstance(f0, torch.Tensor) and f0.is_cuda else torch.device(
+                "cuda", torch.cuda.current_device())
+        as_t = lambda x: torch.as_tensor(np.asarray(x.detach().cpu() if isinstance(x, torch.Tensor) else x),
+                                         dtype=torch.float32).to(device)
+        f0_t, sp_t, ap_t = as_t(f0).reshape(1, -1), as_t(logspc), as_t(codeap)
+        T = f0_t.shape[1]
+        sp_t = sp_t.reshape(1, T, -1)
+        ap_t = ap_t.reshape(1, T, -1)
+        wav, wav_len, status = self.decode_batch(f0_t, sp_t, ap_t)
+        st = int(status[0])
+        if st == K.WORLD_SHORT:
+            raise ValueError("WORLD synthesis needs at least two frames")
+        if st == K.WORLD_NONFINITE:
+            raise ValueError("WORLD synthesis: f0, logspc or codeap holds NaN or inf")
+        return wav[0, :int(wav_len[0])].double().cpu().numpy()
