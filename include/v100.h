@@ -416,6 +416,38 @@ int v100_world_synthesize(const float* f0, int64_t f0_sb, int64_t f0_st, const f
                           void* workspace, float* wav, int64_t wav_pitch, int32_t* wav_len, int32_t* status,
                           void* stream);
 
+/* ------------------------------------------------------------------------------------------------
+ * Resampling
+ * ------------------------------------------------------------------------------------------------ */
+
+/*
+ * Polyphase sinc resampling of a padded batch.  Replaces torchaudio.functional.resample, which
+ * MelSpectrogramAudioTransform.forward applies after load when a file is not at the transform's rate
+ * (voice100/data_modules.py:288-289): torchaudio's _get_sinc_resample_kernel builds a dense [n][1][2w + o] kernel
+ * and _apply_sinc_resample_kernel runs it as a conv1d at stride o.  Rates are reduced by their gcd (o -> n); the
+ * non-zero taps of each phase p form one contiguous run, and only that run is stored:
+ *   out[b][j n + p] = sum_{i < count[p]} taps[off[p] + i] * wav[b][j o + start[p] + i - w]
+ * with wav taken as 0 outside [0, len[b]): padding past a row's length is never read into a result.  Each output is
+ * one fp32 fmaf chain in i order, so the bits do not depend on the batch or the run.
+ *   wav        [B][wav_pitch] samples of `wav_dtype` (V100_WAV_F32 | V100_WAV_I16, int16 scaled by 1/32768);
+ *              len int32 [B] on the device, clamped to [0, L_in], L_in <= wav_pitch
+ *   start, count, off  int32 [n] device arrays: phase p's run is taps[off[p] .. off[p] + count[p]) and covers dense
+ *              kernel columns [start[p], start[p] + count[p]), which must lie in [0, 2w + o) (a run outside it is
+ *              clipped, never read past);  taps fp32 [n_taps]
+ *   out        fp32 [B][out_pitch], L_out <= out_pitch: every sample of [0, L_out) is written; out_len[b] is
+ *              torchaudio's output length for len[b] samples, min(ceil(float32(n len / o)), n (len / o + 1), L_out):
+ *              the float64 quotient rounded to float32 as torch.ceil(torch.as_tensor(...)) does, which is
+ *              ceil(n len / o) until float32 can no longer resolve 1/o (n len / o >= 2^15 at o = 441); samples
+ *              [out_len[b], L_out) are 0
+ *   out_len    optional int32 [B]
+ * Limits (V100_E_UNSUPPORTED beyond them): B <= 65535, n <= 16384 phases, L_in and L_out < 2^31, and the input span
+ * of four frames, 3 o + 2w + o, at most 16384 samples.  One CTA per (tile of output frames, utterance); no host
+ * synchronisation, CUDA-graph capturable.
+ */
+int v100_resample(const void* wav, int wav_dtype, const int32_t* len, int B, int64_t wav_pitch, int64_t L_in,
+                  const int32_t* start, const int32_t* count, const int32_t* off, const float* taps, int n_taps,
+                  int o, int n, int w, float* out, int64_t out_pitch, int64_t L_out, int32_t* out_len, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

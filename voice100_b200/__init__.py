@@ -6,11 +6,12 @@ Drop-in module names follow the reference (kaiidams/voice100):
     voice100.models.tts.TextToAlignTextModel           -> voice100_b200.TextToAlignTextModel
     voice100.models.tts.AlignTextToAudioModel          -> voice100_b200.AlignTextToAudioModel
     voice100.vocoder.WORLDVocoder (decode)             -> voice100_b200.WORLDVocoder
+    torchaudio.functional.resample                     -> voice100_b200.resample
 All compute goes through libv100.so (include/v100.h); importing this package does not need a GPU, but
 every forward does, and fails loudly otherwise.
 """
 from ._lib import V100Error, LIB_PATH  # noqa: F401
-from .data_modules import MelSpectrogramAudioTransform, BLANK_AUDIO, LOG_OFFSET, MELSPEC_DIM  # noqa: F401
+from .data_modules import MelSpectrogramAudioTransform, BLANK_AUDIO, LOG_OFFSET, MELSPEC_DIM, resample  # noqa: F401
 from .asr import AudioToTextCTC, ConvVoiceEncoder, LinearCharDecoder, AsrPipeline  # noqa: F401
 from .tts import (TextToAlignTextModel, AlignTextToAudioModel, VoiceDecoder, WORLDNorm, align_batch,  # noqa: F401
                   TtsPipeline)

@@ -45,6 +45,7 @@ SIGNATURES = {
     "v100_world_workspace_bytes": [_i, _l],   # returns int64 (restype set in lib())
     "v100_world_timebase": [_p, _l, _l, _p, _l, _l, _l, _p, _l, _l, _p, _i, _i, _p, _p, _p, _p],
     "v100_world_synthesize": [_p, _l, _l, _p, _l, _l, _l, _p, _l, _l, _p, _i, _i, _p, _l, _p, _p, _l, _p, _p, _p],
+    "v100_resample": [_p, _i, _p, _i, _l, _l, _p, _p, _p, _p, _i, _i, _i, _i, _p, _l, _l, _p, _p],
 }
 
 ABI_VERSION = 8

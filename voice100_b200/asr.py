@@ -12,6 +12,7 @@ from torch import nn
 
 from . import kernels as K
 from ._lib import V100Error
+from .data_modules import resampled_length
 from .blocks import (InvertedResidualParams, PreparedCache, StorageDtypeMixin, require_eval_cuda,
                      run_inverted_residual)
 from .synth import asr_encoder_blocks
@@ -104,24 +105,33 @@ class AsrPipeline:
     def __init__(self, transform, model: AudioToTextCTC):
         self.transform, self.model = transform, model
 
+    def _rate(self, sample_rate):
+        """The input rate as a resampling key: None when it is the transform's own rate (no resampling)."""
+        return None if sample_rate is None or sample_rate == self.transform.sample_rate else sample_rate
+
     @torch.no_grad()
-    def __call__(self, waveform: torch.Tensor, lengths: torch.Tensor) -> Tuple[torch.Tensor, torch.Tensor]:
+    def __call__(self, waveform: torch.Tensor, lengths: torch.Tensor,
+                 sample_rate: Optional[int] = None) -> Tuple[torch.Tensor, torch.Tensor]:
         """device waveform fp32 or int16 PCM [B, L], lengths [B] -> (tokens int64 [B, T'], valid lengths int32 [B]).
         Three kinds of kernel and nothing else: log-mel (also emits audio_len), the conv stack, the CTC tail (also
-        emits output_length)."""
-        feats, audio_len = self.transform.logmel_batch(waveform, lengths, ncw_dtype=self.model.storage_dtype)
+        emits output_length).  `sample_rate` is the waveform's rate (None = the transform's); any other rate is
+        resampled on the device first (one more kernel: MelSpectrogramAudioTransform.logmel_batch(orig_freq=...))."""
+        feats, audio_len = self.transform.logmel_batch(waveform, lengths, ncw_dtype=self.model.storage_dtype,
+                                                       orig_freq=self._rate(sample_rate))
         return self.model.greedy(feats, audio_len)
 
     @torch.no_grad()
-    def transcribe_ids(self, waveform: torch.Tensor, lengths: torch.Tensor, blank: int = 0):
+    def transcribe_ids(self, waveform: torch.Tensor, lengths: torch.Tensor, blank: int = 0,
+                       sample_rate: Optional[int] = None):
         """waveform -> CTC-collapsed token ids on the device: (ids int64 [B, T'] blank-padded, counts int32 [B]).
         `tokenizer.decode(ids[b, :counts[b]])` is then the final text (no merge_repeated pass needed)."""
-        tokens, out_len = self(waveform, lengths)
+        tokens, out_len = self(waveform, lengths, sample_rate=sample_rate)
         return K.ctc_collapse(tokens, out_len, blank)
 
     @torch.no_grad()
-    def _capture(self, batch: int, samples: int, dev, wav_dtype=torch.float32):
-        """-> (graph, static waveform, static lengths, static tokens, static out_len) for one fixed shape."""
+    def _capture(self, batch: int, samples: int, dev, wav_dtype=torch.float32, sample_rate=None):
+        """-> (graph, static waveform, static lengths, static tokens, static out_len) for one fixed shape.  With a
+        `sample_rate` the resampled buffer inside the graph is [batch, ceil(n samples / o)]."""
         with torch.cuda.device(dev):
             wav_s = torch.zeros((batch, samples), dtype=wav_dtype, device=dev)
             len_s = torch.full((batch,), samples, dtype=torch.int32, device=dev)
@@ -129,23 +139,25 @@ class AsrPipeline:
             side.wait_stream(torch.cuda.current_stream(dev))
             with torch.cuda.stream(side):          # warm-up outside capture: one-time function attributes, caches
                 for _ in range(2):
-                    self(wav_s, len_s)
+                    self(wav_s, len_s, sample_rate=sample_rate)
             torch.cuda.current_stream(dev).wait_stream(side)
             graph = torch.cuda.CUDAGraph()
             with torch.cuda.graph(graph):
-                tok_s, out_s = self(wav_s, len_s)
+                tok_s, out_s = self(wav_s, len_s, sample_rate=sample_rate)
         return graph, wav_s, len_s, tok_s, out_s
 
     @torch.no_grad()
-    def graphed(self, batch: int, samples: int, device="cuda", wav_dtype=torch.float32):
+    def graphed(self, batch: int, samples: int, device="cuda", wav_dtype=torch.float32,
+                sample_rate: Optional[int] = None):
         """Capture the whole path (log-mel -> encoder -> head -> argmax: 30 launches, all libv100 kernels) for one
         fixed [batch, samples] shape into a CUDA graph.  Replaying it removes the per-launch gaps: 8-10 % at
         256 x 15 s, 2.5x at 8 x 10 s (which is ~0.3 ms of GPU work behind ~0.7 ms of launches).
-        `wav_dtype` torch.float32 or torch.int16 (PCM).  Returns `run(waveform, lengths) -> (tokens, out_len)`; the
-        outputs are static buffers overwritten by the next replay; `run.graph.replay()` re-runs on the current
+        `wav_dtype` torch.float32 or torch.int16 (PCM).  `sample_rate` is the input's rate (None = the transform's);
+        another rate adds the resampling kernel to the graph.  Returns `run(waveform, lengths) -> (tokens, out_len)`;
+        the outputs are static buffers overwritten by the next replay; `run.graph.replay()` re-runs on the current
         contents of `run.waveform/.lengths`."""
         dev = torch.device(device)
-        graph, wav_s, len_s, tok_s, out_s = self._capture(batch, samples, dev, wav_dtype)
+        graph, wav_s, len_s, tok_s, out_s = self._capture(batch, samples, dev, wav_dtype, self._rate(sample_rate))
 
         def run(waveform: torch.Tensor, lengths: torch.Tensor):
             wav_s.copy_(waveform, non_blocking=True)
@@ -156,7 +168,8 @@ class AsrPipeline:
         return run
 
     @torch.no_grad()
-    def submit_host(self, waveform: torch.Tensor, lengths: torch.Tensor, device="cuda", chunks: int = 4):
+    def submit_host(self, waveform: torch.Tensor, lengths: torch.Tensor, device="cuda", chunks: int = 4,
+                    sample_rate: Optional[int] = None):
         """Asynchronous end-to-end call: host buffers in (pin them for full PCIe speed), host tokens out.
         `waveform` is fp32 or int16 PCM (half the H2D bytes; identical features for 16-bit sources).
         The batch is cut into `chunks` groups of utterances; each group has its own captured CUDA graph with
@@ -166,7 +179,9 @@ class AsrPipeline:
         uploading) before the previous one has finished computing.  Two tickets may be in flight: consecutive
         calls alternate between two sets of graphs / device buffers, so batch i+1 uploads into its own buffers
         while batch i still computes.  `chunks=1` gives the best throughput (whole-batch kernels, uploads hidden
-        behind the previous batch), more chunks give a shorter latency for a single batch."""
+        behind the previous batch), more chunks give a shorter latency for a single batch.
+        `sample_rate` is the input's rate (None = the transform's); another rate is resampled inside each graph, so
+        the upload stays at the input's size."""
         dev = torch.device(device)
         if dev.index is None:
             dev = torch.device("cuda", torch.cuda.current_device())
@@ -175,7 +190,9 @@ class AsrPipeline:
         if getattr(self, "_copy_stream", None) is None or self._copy_stream.device != dev:
             self._copy_stream = torch.cuda.Stream(dev)
             self._host_out, self._slot, self._chunk_graphs = {}, 0, {}
-        T_out = (self.transform.num_frames(L) + 1) // 2
+        rate = self._rate(sample_rate)
+        L_feat = L if rate is None else resampled_length(L, rate, self.transform.sample_rate)
+        T_out = (self.transform.num_frames(L_feat) + 1) // 2
         slot = self._slot
         key = (B, T_out, slot)
         self._slot ^= 1                      # double-buffered device inputs and pinned outputs: two tickets in flight
@@ -188,9 +205,9 @@ class AsrPipeline:
             staged = []
             for i in range(n):
                 a, b = B * i // n, B * (i + 1) // n
-                gkey = (i, b - a, L, slot, waveform.dtype)
+                gkey = (i, b - a, L, slot, waveform.dtype, rate)
                 if gkey not in self._chunk_graphs:
-                    self._chunk_graphs[gkey] = list(self._capture(b - a, L, dev, waveform.dtype)) + [None]
+                    self._chunk_graphs[gkey] = list(self._capture(b - a, L, dev, waveform.dtype, rate)) + [None]
                 cg = self._chunk_graphs[gkey]
                 graph, wav_s, len_s, tok_s, out_s, done = cg
                 with torch.cuda.stream(self._copy_stream):
@@ -213,9 +230,10 @@ class AsrPipeline:
             done_all.record(cur)
         return _Ticket(done_all, tok_h, len_h)
 
-    def transcribe_host(self, waveform: torch.Tensor, lengths: torch.Tensor, device="cuda", chunks: int = 4):
+    def transcribe_host(self, waveform: torch.Tensor, lengths: torch.Tensor, device="cuda", chunks: int = 4,
+                        sample_rate: Optional[int] = None):
         """Synchronous form of submit_host -> (tokens int64 [B, T'] pinned host tensor, valid lengths [B])."""
-        return self.submit_host(waveform, lengths, device, chunks).result()
+        return self.submit_host(waveform, lengths, device, chunks, sample_rate).result()
 
 
 class _Ticket:

@@ -273,4 +273,11 @@ int v100_world_synthesize(const float* f0, int64_t f0_sb, int64_t f0_st, const f
                           noise_len, workspace, wav, wav_pitch, wav_len, status, STREAM(stream));
 }
 
+int v100_resample(const void* wav, int wav_dtype, const int32_t* len, int B, int64_t wav_pitch, int64_t L_in,
+                  const int32_t* start, const int32_t* count, const int32_t* off, const float* taps, int n_taps,
+                  int o, int n, int w, float* out, int64_t out_pitch, int64_t L_out, int32_t* out_len, void* stream) {
+  return resample(wav, wav_dtype, len, B, wav_pitch, L_in, start, count, off, taps, n_taps, o, n, w, out, out_pitch,
+                  L_out, out_len, STREAM(stream));
+}
+
 }  // extern "C"

@@ -620,3 +620,28 @@ def world_synthesize(f0: torch.Tensor, logspc: torch.Tensor, codeap: torch.Tenso
     _call(f0, "v100_world_synthesize", *_world_args(f0, logspc, codeap, frame_len), B, T, noise.data_ptr(),
           noise.numel(), ws.data_ptr(), wav.data_ptr(), Y, out[0].data_ptr(), out[1].data_ptr())
     return wav, out[0], out[1]
+
+
+# ---------------------------------------------------------------------------------------------- resampling
+
+
+def resample(wav: torch.Tensor, lengths: torch.Tensor, table, L_out: int):
+    """One v100_resample call.  wav fp32 or int16 PCM [B, L] with unit stride along time and any row pitch; lengths
+    int32 [B] on the device; table a data_modules.ResampleTable on the same device.
+    -> (out fp32 [B, L_out], out_len int32 [B] = min(ceil(n lengths / o), L_out)); no host synchronisation."""
+    _cuda(lengths, torch.int32)
+    if wav.dtype not in (torch.float32, torch.int16):
+        raise _lib.V100Error(f"waveforms must be float32 or int16 PCM, got {wav.dtype}")
+    if not wav.is_cuda or wav.dim() != 2 or wav.stride(1) != 1:
+        raise _lib.V100Error("resample: wav must be a CUDA [B, L] tensor with unit stride along time")
+    _same_device(wav, lengths, table.taps)
+    B, L = wav.shape
+    pitch = wav.stride(0) if B > 1 else L
+    out = torch.empty((B, L_out), device=wav.device, dtype=torch.float32)
+    out_len = torch.empty((B,), device=wav.device, dtype=torch.int32)
+    if B == 0:
+        return out, out_len
+    _call(wav, "v100_resample", wav.data_ptr(), 1 if wav.dtype == torch.int16 else 0, lengths.data_ptr(), B, pitch, L,
+          table.start.data_ptr(), table.count.data_ptr(), table.off.data_ptr(), _ptr(table.taps), table.taps.numel(),
+          table.o, table.n, table.width, out.data_ptr(), L_out, L_out, out_len.data_ptr())
+    return out, out_len

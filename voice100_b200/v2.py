@@ -14,7 +14,7 @@ is one persistent kernel per layer (v100_lstm_layer).
 """
 from __future__ import annotations
 
-from typing import List, Sequence, Tuple
+from typing import List, Optional, Sequence, Tuple
 
 import torch
 from torch import nn
@@ -248,8 +248,9 @@ class AsrV2Pipeline(AsrPipeline):
         self.transform, self.model = transform, model
 
     @torch.no_grad()
-    def __call__(self, waveform: torch.Tensor, lengths: torch.Tensor):
-        feats, audio_len = self.transform.logmel_batch(waveform, lengths, ncw_dtype=self.model.storage_dtype)
+    def __call__(self, waveform: torch.Tensor, lengths: torch.Tensor, sample_rate: Optional[int] = None):
+        feats, audio_len = self.transform.logmel_batch(waveform, lengths, ncw_dtype=self.model.storage_dtype,
+                                                       orig_freq=self._rate(sample_rate))
         tokens, x_len = self.model.greedy(feats, audio_len)
         return tokens.t().contiguous(), x_len
 
