@@ -417,6 +417,48 @@ int v100_world_synthesize(const float* f0, int64_t f0_sb, int64_t f0_st, const f
                           void* stream);
 
 /* ------------------------------------------------------------------------------------------------
+ * WORLD analysis (fs = 16000, frame period 10 ms, fft_size 512)
+ *
+ * Replaces WORLDVocoder.encode (voice100/vocoder.py:66-88): pyworld.dio (f0_floor 71, f0_ceil 800, 2 channels an
+ * octave, speed 1, allowed range 0.1), stonemask, cheaptrick (fft_size 512), d4c (threshold 0.85),
+ * code_aperiodicity, then logspc = log(sp + 1e-15), run on the host one utterance at a time.  The contract is the
+ * float64 restatement oracle/world_analysis.py; parity with pyworld itself has not been checked (DESIGN.md section
+ * 3.10 lists the conventions a restatement could have wrong).  Status codes are V100_WORLD_*: V100_WORLD_SHORT for
+ * fewer than 4 frames (L < 480 samples, where FixF0Contour returns early), V100_WORLD_NONFINITE for a NaN or inf
+ * sample.
+ * ------------------------------------------------------------------------------------------------ */
+
+/*
+ * Bytes of the workspace of v100_world_analyze for B utterances of at most L_max samples (vocoder.py:66-88).  It
+ * depends on the shapes only; it is dominated by the refined zero crossings, 28 series of at most L_max / 2 + 1
+ * float64 values per utterance (about 112 bytes a sample).
+ */
+int64_t v100_world_analysis_workspace_bytes(int B, int64_t L_max);
+
+/*
+ * WORLD analysis of a padded batch (vocoder.py:66-88): Dio + StoneMask + CheapTrick + D4C + CodeAperiodicity.
+ *   wav        [B][wav_pitch] fp32 (wav_dtype 0) or int16 PCM (wav_dtype 1, scaled by 1 / 32768), unit stride along
+ *              time; utterance b is wav[b][0, min(max(len[b], 0), L_max))
+ *   taps       float64 [1633] on the device: DIO's low-cut filter (641 taps: w[i] = 0.5 - 0.5 cos(2 pi (i + 1) / 642),
+ *              h = -w / sum(w), h[320] += 1), then the Nuttall windows of the 7 bands (320, 224, 160, 112, 80, 56, 40
+ *              taps: 0.355768 - 0.487396 cos(2 pi u) + 0.144232 cos(4 pi u) - 0.012604 cos(6 pi u), u = i / (n - 1)),
+ *              as the restatement's dio_taps() computes them
+ *   noise      v100_world_noise output with noise_len >= 5290 (L_max / 160 + 1) values (CheapTrick's and D4C's dither)
+ *   workspace  v100_world_analysis_workspace_bytes(B, L_max) bytes, 256-byte aligned
+ *   T          frames of the outputs, T >= L_max / 160 + 1
+ *   f0         fp32 [B][T] (Hz, 0 = unvoiced), logspc fp32 [B][T][257] (log(sp + 1e-15)), codeap fp32 [B][T]
+ *              (20 log10 of the aperiodicity at 3000 Hz); every element is written, rows at or past frame_len[b] are 0
+ *   frame_len  int32 [B]: len / 160 + 1 (0 for a rejected utterance);  status  int32 [B]: V100_WORLD_*
+ * All float64.  The DIO stage (filters, crossings, contour, FixF0Contour) repeats the restatement's operations in its
+ * order without FMA contraction, so its f0 contour is bit-identical to it.  Deterministic: an utterance's outputs do
+ * not depend on the rest of the batch.  No host synchronisation; CUDA-graph capturable.  L_max above 2^30, or B or T
+ * above 65535, is V100_E_UNSUPPORTED.
+ */
+int v100_world_analyze(const void* wav, int wav_dtype, int64_t wav_pitch, const int32_t* len, int B, int64_t L_max,
+                       const double* taps, const double* noise, int64_t noise_len, void* workspace, int T, float* f0,
+                       float* logspc, float* codeap, int32_t* frame_len, int32_t* status, void* stream);
+
+/* ------------------------------------------------------------------------------------------------
  * Resampling
  * ------------------------------------------------------------------------------------------------ */
 

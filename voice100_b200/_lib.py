@@ -46,6 +46,8 @@ SIGNATURES = {
     "v100_world_timebase": [_p, _l, _l, _p, _l, _l, _l, _p, _l, _l, _p, _i, _i, _p, _p, _p, _p],
     "v100_world_synthesize": [_p, _l, _l, _p, _l, _l, _l, _p, _l, _l, _p, _i, _i, _p, _l, _p, _p, _l, _p, _p, _p],
     "v100_resample": [_p, _i, _p, _i, _l, _l, _p, _p, _p, _p, _i, _i, _i, _i, _p, _l, _l, _p, _p],
+    "v100_world_analysis_workspace_bytes": [_i, _l],   # returns int64 (restype set in lib())
+    "v100_world_analyze": [_p, _i, _l, _p, _i, _l, _p, _p, _l, _p, _i, _p, _p, _p, _p, _p, _p],
 }
 
 ABI_VERSION = 8
@@ -71,6 +73,7 @@ def lib():
         handle.v100_lstm_workspace_bytes.argtypes = [_i, _i]
         handle.v100_lstm_workspace_bytes.restype = _l
         handle.v100_world_workspace_bytes.restype = _l
+        handle.v100_world_analysis_workspace_bytes.restype = _l
         handle.v100_last_error.argtypes = []
         handle.v100_last_error.restype = C.c_char_p
         if handle.v100_abi_version() != ABI_VERSION:
@@ -87,6 +90,9 @@ KERNELS_PER_CALL["v100_conv1d"] = 2   # tap stacking + GEMM
 KERNELS_PER_CALL["v100_abi_version"] = 0
 KERNELS_PER_CALL["v100_world_synthesize"] = 2   # time base + synthesis
 KERNELS_PER_CALL["v100_world_workspace_bytes"] = 0
+KERNELS_PER_CALL["v100_world_analysis_workspace_bytes"] = 0
+KERNELS_PER_CALL["v100_world_analyze"] = 13     # prep, low-cut, bands x2, scan, contour, fix, StoneMask, draws x2,
+                                                # CheapTrick, LoveTrain, D4C
 
 stats = {"launches": 0}
 tracer = None  # optional object with before(name)/after(name), used by bench.py for per-kernel CUDA events

@@ -273,6 +273,15 @@ int v100_world_synthesize(const float* f0, int64_t f0_sb, int64_t f0_st, const f
                           noise_len, workspace, wav, wav_pitch, wav_len, status, STREAM(stream));
 }
 
+int64_t v100_world_analysis_workspace_bytes(int B, int64_t L_max) { return world_analysis_workspace_bytes(B, L_max); }
+
+int v100_world_analyze(const void* wav, int wav_dtype, int64_t wav_pitch, const int32_t* len, int B, int64_t L_max,
+                       const double* taps, const double* noise, int64_t noise_len, void* workspace, int T, float* f0,
+                       float* logspc, float* codeap, int32_t* frame_len, int32_t* status, void* stream) {
+  return world_analyze(wav, wav_dtype, wav_pitch, len, B, L_max, taps, noise, noise_len, workspace, T, f0, logspc,
+                       codeap, frame_len, status, STREAM(stream));
+}
+
 int v100_resample(const void* wav, int wav_dtype, const int32_t* len, int B, int64_t wav_pitch, int64_t L_in,
                   const int32_t* start, const int32_t* count, const int32_t* off, const float* taps, int n_taps,
                   int o, int n, int w, float* out, int64_t out_pitch, int64_t L_out, int32_t* out_len, void* stream) {

@@ -122,6 +122,13 @@ int world_synthesize(const float* f0, int64_t f0_sb, int64_t f0_st, const float*
                      const int32_t* frame_len, int B, int T, const double* noise, int64_t noise_len, void* workspace,
                      float* wav, int64_t wav_pitch, int32_t* wav_len, int32_t* status, cudaStream_t stream);
 
+// WORLD analysis (world_analysis.cu)
+int64_t world_analysis_workspace_bytes(int B, int64_t L_max);
+int64_t world_analysis_noise_values(int64_t L_max);
+int world_analyze(const void* wav, int wav_dtype, int64_t wav_pitch, const int32_t* len, int B, int64_t L_max,
+                  const double* taps, const double* noise, int64_t noise_len, void* workspace, int T, float* f0,
+                  float* logspc, float* codeap, int32_t* frame_len, int32_t* status, cudaStream_t stream);
+
 // Resampling (resample.cu)
 int resample(const void* wav, int wav_dtype, const int32_t* len, int B, int64_t wav_pitch, int64_t L_in,
              const int32_t* start, const int32_t* count, const int32_t* off, const float* taps, int n_taps, int o,

@@ -622,6 +622,83 @@ def world_synthesize(f0: torch.Tensor, logspc: torch.Tensor, codeap: torch.Tenso
     return wav, out[0], out[1]
 
 
+# ---------------------------------------------------------------------------------------------- WORLD analysis
+
+_WORLD_ANALYSIS_DRAWS = 5290                          # dither values a frame can read (LoveTrain + D4C), per frame
+_dio_taps = {}                                        # device index -> float64 DIO filter table
+
+
+def dio_taps(device) -> torch.Tensor:
+    """DIO's filters as v100_world_analyze reads them (float64 [1633]): the 641-tap low-cut filter, then the Nuttall
+    windows of the 7 bands.  Built with numpy, by the same expressions as oracle/world_analysis.py's dio_taps(), once
+    per device and outside graph capture."""
+    import numpy as np
+    dev = torch.device(device)
+    if dev.index is None:
+        dev = torch.device("cuda", torch.cuda.current_device())
+    tab = _dio_taps.get(dev.index)
+    if tab is None:
+        if torch.cuda.is_current_stream_capturing():
+            raise _lib.V100Error("the DIO filter table is built on first use: run world_analyze once before capture")
+        pi = 3.1415926535897932384
+        i = np.arange(1, 642, dtype=np.float64)
+        w = 0.5 - 0.5 * np.cos(i * 2.0 * pi / 642)
+        s = 0.0
+        for v in w:
+            s += v
+        low = -w / s
+        low[320] += 1.0
+        parts = [low]
+        for k in range(7):
+            x = 16000 / (71.0 * 2.0 ** ((k + 1) / 2.0)) / 2.0
+            n = 4 * int(x + 0.5)
+            u = np.arange(n, dtype=np.float64) / (n - 1.0)
+            parts.append(0.355768 - 0.487396 * np.cos(2.0 * pi * u) + 0.144232 * np.cos(4.0 * pi * u)
+                         - 0.012604 * np.cos(6.0 * pi * u))
+        tab = torch.from_numpy(np.concatenate(parts)).to(dev)
+        _dio_taps[dev.index] = tab
+    return tab
+
+
+def world_analyze(wav: torch.Tensor, lengths: torch.Tensor, T: int = None):
+    """WORLD analysis on the device (v100_world_analyze): Dio + StoneMask + CheapTrick + D4C + CodeAperiodicity at
+    16 kHz, 10 ms frames, fft_size 512, for a padded batch.  wav fp32 or int16 PCM [B, L] with unit stride along time
+    and any row pitch; lengths int32 [B] on the device.
+    -> (f0 fp32 [B, T], logspc fp32 [B, T, 257], codeap fp32 [B, T, 1], frame_len int32 [B] = lengths // 160 + 1,
+    status int32 [B] = WORLD_*), T = L // 160 + 1 by default.  Rows at and past frame_len are 0; a rejected utterance
+    (WORLD_SHORT: fewer than 480 samples, WORLD_NONFINITE: a NaN or inf sample) is all 0 with frame_len 0.  No host
+    synchronisation; capturable once this device's noise and filter tables exist (a first call builds them)."""
+    _cuda(lengths, torch.int32)
+    if wav.dtype not in (torch.float32, torch.int16):
+        raise _lib.V100Error(f"world_analyze: waveforms must be float32 or int16 PCM, got {wav.dtype}")
+    if not wav.is_cuda or wav.dim() != 2 or wav.stride(1) != 1:
+        raise _lib.V100Error("world_analyze: wav must be a CUDA [B, L] tensor with unit stride along time")
+    B, L = wav.shape
+    if tuple(lengths.shape) != (B,):
+        raise _lib.V100Error(f"world_analyze: lengths must be int32 [{B}]")
+    _same_device(wav, lengths)
+    if B <= 0:
+        raise _lib.V100Error("world_analyze: empty batch")
+    T = L // WORLD_HOP + 1 if T is None else int(T)
+    if T < L // WORLD_HOP + 1:
+        raise _lib.V100Error(f"world_analyze: T = {T} frames < L // 160 + 1 = {L // WORLD_HOP + 1}")
+    dev = wav.device
+    noise = world_noise(_WORLD_ANALYSIS_DRAWS * (L // WORLD_HOP + 1), dev)
+    taps = dio_taps(dev)
+    n = int(_lib.lib().v100_world_analysis_workspace_bytes(B, L))
+    ws = torch.empty((n + 256,), device=dev, dtype=torch.uint8)
+    off = (-ws.data_ptr()) % 256
+    f0 = torch.empty((B, T), device=dev, dtype=torch.float32)
+    logspc = torch.empty((B, T, WORLD_BINS), device=dev, dtype=torch.float32)
+    codeap = torch.empty((B, T, 1), device=dev, dtype=torch.float32)
+    out = torch.empty((2, B), device=dev, dtype=torch.int32)
+    pitch = wav.stride(0) if B > 1 else L
+    _call(wav, "v100_world_analyze", wav.data_ptr(), 1 if wav.dtype == torch.int16 else 0, pitch, lengths.data_ptr(),
+          B, L, taps.data_ptr(), noise.data_ptr(), noise.numel(), ws.data_ptr() + off, T, f0.data_ptr(),
+          logspc.data_ptr(), codeap.data_ptr(), out[0].data_ptr(), out[1].data_ptr())
+    return f0, logspc, codeap, out[0], out[1]
+
+
 # ---------------------------------------------------------------------------------------------- resampling
 
 

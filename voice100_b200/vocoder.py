@@ -5,8 +5,9 @@ The reference's shipped TTS config trains AlignTextToAudio on 25 mel-cepstral co
 (voice100/export_onnx.py:81-97 `AlignTextToAudioPredict`, voice100/vocoder.py:115-123 `create_mc2sp_matrix`).
 Un-normalisation and that matrix are both linear, so here they are folded into the projection layer: the head GEMM
 emits the 257 log-spectrum bins directly and the conversion costs nothing at run time.
-WORLD waveform synthesis (the reference's WORLDVocoder.decode, pyworld on the host) runs on the device through
-`WORLDVocoder` (v100_world_synthesize); WORLD analysis (encode) is not on the inference path and stays out of scope.
+The WORLD vocoder runs on the device through `WORLDVocoder`, both halves of the reference's class: synthesis
+(`decode`, pyworld.decode_aperiodicity + synthesize: v100_world_synthesize) and analysis (`encode`, pyworld.dio +
+stonemask + cheaptrick + d4c + code_aperiodicity, the targets every TTS model here trains on: v100_world_analyze).
 """
 from __future__ import annotations
 
@@ -103,11 +104,13 @@ class AlignTextToAudioPredict(nn.Module):
 
 
 class WORLDVocoder:
-    """WORLD synthesis on the device, in place of the reference's WORLDVocoder.decode (voice100/vocoder.py:89-102:
-    pyworld.decode_aperiodicity + pyworld.synthesize, one utterance on a CPU core).  Only the configuration every model
-    here emits is implemented: 16 kHz, 10 ms frames, 512-point FFT (257 log-spectrum bins, one coded-aperiodicity band).
-    The algorithm is the restatement in oracle/world.py; parity with pyworld itself is unverified (DESIGN.md 3.8).
-    Inputs are used as fp32, the precision the models produce them in."""
+    """The WORLD vocoder on the device, in place of the reference's WORLDVocoder (voice100/vocoder.py): `decode`
+    (vocoder.py:89-102, pyworld.decode_aperiodicity + pyworld.synthesize) and `encode` (vocoder.py:66-88, pyworld.dio +
+    stonemask + cheaptrick + d4c + code_aperiodicity), each one utterance on a CPU core in the reference.  Only the
+    configuration every model here uses is implemented: 16 kHz, 10 ms frames, 512-point FFT (257 log-spectrum bins,
+    one coded-aperiodicity band).  The algorithms are the restatements in oracle/world.py and oracle/world_analysis.py;
+    parity with pyworld itself is unverified (DESIGN.md 3.8 and 3.10).  Synthesis inputs are used as fp32, the
+    precision the models produce them in."""
 
     def __init__(self, sample_rate: int = 16000, frame_period: float = 10.0, n_fft: int = 512) -> None:
         if (sample_rate, float(frame_period), n_fft) != (K.WORLD_FS, 10.0, K.WORLD_FFT):
@@ -143,3 +146,36 @@ class WORLDVocoder:
         if st == K.WORLD_NONFINITE:
             raise ValueError("WORLD synthesis: f0, logspc or codeap holds NaN or inf")
         return wav[0, :int(wav_len[0])].double().cpu().numpy()
+
+    def encode_batch(self, wav: torch.Tensor, wav_len: torch.Tensor, sample_rate: int = None):
+        """WORLD analysis of a padded batch: wav fp32 or int16 PCM [B, L] on the device (unit stride along time, any
+        row pitch), wav_len int [B] -> (f0 fp32 [B, T], logspc fp32 [B, T, 257], codeap fp32 [B, T, 1], frame_len
+        int32 [B], status int32 [B]) as device tensors; see kernels.world_analyze.  A `sample_rate` other than 16000
+        resamples first (voice100_b200.resample, torchaudio's semantics), in the same stream.  No host sync."""
+        wav_len = wav_len.to(device=wav.device, dtype=torch.int32).contiguous()
+        if sample_rate is not None and int(sample_rate) != self.sample_rate:
+            from .data_modules import resample
+            wav, wav_len = resample(wav, int(sample_rate), self.sample_rate, lengths=wav_len)
+        return K.world_analyze(wav, wav_len)
+
+    def encode(self, waveform, device=None):
+        """One 16 kHz utterance, like the reference: waveform [L] (numpy array or tensor, fp32 or int16 PCM)
+        -> float64 numpy (f0 [T], logspc [T, 257], codeap [T, 1]), T = L // 160 + 1.  Runs on `device` (default: the
+        tensor's CUDA device, else the current one).  Raises ValueError for fewer than 480 samples or a NaN / inf."""
+        if device is None:
+            device = waveform.device if isinstance(waveform, torch.Tensor) and waveform.is_cuda else torch.device(
+                "cuda", torch.cuda.current_device())
+        x = waveform.detach().cpu() if isinstance(waveform, torch.Tensor) else torch.from_numpy(np.asarray(waveform))
+        if x.dtype != torch.int16:
+            x = x.to(torch.float32)
+        x = x.reshape(1, -1).contiguous().to(device)
+        f0, logspc, codeap, frame_len, status = self.encode_batch(
+            x, torch.tensor([x.shape[1]], dtype=torch.int32, device=device))
+        st = int(status[0])
+        if st == K.WORLD_SHORT:
+            raise ValueError("WORLD analysis needs at least 480 samples (4 frames)")
+        if st == K.WORLD_NONFINITE:
+            raise ValueError("WORLD analysis: the waveform holds NaN or inf")
+        n = int(frame_len[0])
+        return (f0[0, :n].double().cpu().numpy(), logspc[0, :n].double().cpu().numpy(),
+                codeap[0, :n].double().cpu().numpy())
