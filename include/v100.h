@@ -30,7 +30,7 @@
 extern "C" {
 #endif
 
-#define V100_ABI_VERSION 8
+#define V100_ABI_VERSION 9
 
 #define V100_E_INVALID   (-1)   /* bad argument (null pointer, misaligned pitch, size <= 0)   */
 #define V100_E_UNSUPPORTED (-2) /* shape outside what the kernels implement                   */
@@ -134,22 +134,6 @@ int v100_conv1x1_f32out(const void* x, int64_t x_pitch, const void* W, const flo
 int v100_dwconv1d(const void* x, int64_t x_pitch, const void* w, const float* scale,
                   const float* shift, void* y, int64_t y_pitch,
                   int B, int C, int T_in, int k, int stride, int act, int dtype, void* stream);
-
-/*
- * Block-level fusion of InvertedResidual's first two stages (voice100/models/asr.py:47-49): pointwise expand
- * (1x1 conv + BN + ReLU6, C_in -> H) and depthwise conv (k taps, stride 1, + BN + ReLU6) in ONE kernel:
- *   h[b][c][t] = relu6(scale1[c] * sum_ci W1[c][ci] x[b][ci][t] + shift1[c])        (rounded to `dtype`, on chip only)
- *   y[b][c][o] = relu6(scale2[c] * sum_j wd[c][j] h[b][c][o + j - (k-1)/2] + shift2[c])   zero padded
- * The H-wide tensor h stays in tensor memory / shared memory (a tcgen05 GEMM whose epilogue runs the depthwise FIR on
- * a sliding window of its own output), so it is neither written to nor read back from HBM.  Same numerical contract as
- * v100_conv1x1 followed by v100_dwconv1d.  H % 256 == 0, C_in % 8 == 0, k odd <= 83.
- *   dw_pairs  uint32 [H][128]: the depthwise filter wd [H][k] packed by v100_dw_pack_pairs (zero-extended taps as
- *             adjacent 16-bit pairs, the layout the tensor-core FIR reads its Toeplitz fragments from)
- */
-int v100_dw_pack_pairs(const void* wd, uint32_t* dw_pairs, int C, int k, void* stream);
-int v100_expand_dw(const void* x, int64_t x_pitch, const void* W1, const float* scale1, const float* shift1,
-                   const uint32_t* dw_pairs, const float* scale2, const float* shift2, void* y, int64_t y_pitch,
-                   int B, int C_in, int H, int T, int k, int dtype, void* stream);
 
 /* Same contract, always the plain CUDA-core kernel (any stride).  Used for stride != 1 internally;
  * exported so the tests can cross-check the tensor-core kernel against it on the device. */

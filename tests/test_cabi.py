@@ -23,7 +23,7 @@ def header_functions():
     return {name: [a.strip() for a in args.split(",")] if args.strip() != "void" else [] for name, args in decls}
 
 
-def test_library_loads_and_exports_header_symbols():
+def test_library_loads_exports_header_symbols_and_abi_version():
     from voice100_b200 import build
     build.build()
     assert os.path.exists(_lib.LIB_PATH)
@@ -35,7 +35,7 @@ def test_library_loads_and_exports_header_symbols():
     out = subprocess.run(["nm", "-D", "--defined-only", _lib.LIB_PATH], capture_output=True, text=True).stdout
     exported = set(re.findall(r" T (v100_\w+)", out))
     assert exported == set(funcs), exported ^ set(funcs)
-    assert _lib.lib().v100_abi_version() == _lib.ABI_VERSION == 8
+    assert _lib.lib().v100_abi_version() == _lib.ABI_VERSION == 9
 
 
 def test_plain_c_consumer_compiles_links_and_fails_loudly(tmp_path):

@@ -251,56 +251,6 @@ def test_dwconv_stride2_polyphase_matches_torch(k, T, dtype):
 
 
 # ------------------------------------------------------------------------------------------------
-# fused expand + depthwise (tcgen05 GEMM whose epilogue runs the depthwise FIR on a shared-memory sliding window)
-# ------------------------------------------------------------------------------------------------
-@pytest.mark.parametrize("B,C_in,H,T,k", [
-    (3, 256, 1024, 751, 19),     # asr_en_base blocks 1-3 shape (three time tiles, ragged last tile)
-    (2, 512, 2048, 751, 83),     # block 8: the longest filter, Q = 7
-    (2, 512, 2048, 300, 59),
-    (5, 256, 1024, 256, 35),     # T a multiple of the tile: the flush pass produces the last p outputs
-    (2, 256, 1024, 257, 51),     # one column into the second tile
-    (3, 128, 512, 41, 27),       # shorter than the filter
-    (2, 64, 256, 100, 11),       # one k-block, Q = 2
-    (2, 72, 512, 333, 67),       # C_in not a multiple of 64
-    (1, 256, 1024, 1, 7),        # a single frame
-    (150, 64, 256, 130, 33),     # more units than CTA pairs: the persistent loop recycles window and TMEM buffers
-])
-@pytest.mark.parametrize("dtype", DTYPES)
-def test_expand_dw_fused_matches_torch_and_unfused(B, C_in, H, T, k, dtype):
-    x = rnd(B, C_in, T, seed=41)
-    W1 = rnd(H, C_in, seed=42, scale=1.0 / math.sqrt(C_in)).to(dtype)
-    wd = rnd(H, k, seed=43, scale=1.0 / math.sqrt(k)).to(dtype)
-    s1, b1 = torch.rand(H, device=DEV) + 0.5, rnd(H, seed=44) + 1.0
-    s2, b2 = torch.rand(H, device=DEV) + 0.5, rnd(H, seed=45) + 1.0
-    xn = ncw(x, dtype)
-    y = K.expand_dw(xn, W1, s1, b1, K.dw_pack_pairs(wd), s2, b2, k)
-    h = K.conv1x1(xn, W1, s1, b1, K.ACT_RELU6)
-    y2 = K.dwconv(h, wd, s2, b2, k, 1, K.ACT_RELU6)
-    torch.cuda.synchronize()
-    assert y.T == T and y.C == H
-    # fp32 PyTorch on the same 16-bit operands, with the hidden tensor rounded to the storage type (the contract)
-    href = (F.conv1d(xn.valid().float(), W1.float()[:, :, None]) * s1[None, :, None] + b1[None, :, None]).clamp(0, 6)
-    href = href.to(dtype).float()
-    ref = (F.conv1d(href, wd.float()[:, None, :], padding=(k - 1) // 2, groups=H) * s2[None, :, None] + b2[None, :, None]).clamp(0, 6)
-    assert rel_err(y.valid().float(), ref) < OUT_TOL[dtype]
-    # ... and the three-kernel path: same operands, same contract; only the fp32 summation order inside the FIR differs
-    d = (y.valid().float() - y2.valid().float()).abs()
-    assert float(d.max()) <= 6.0 * (2.0 ** -7 if dtype == torch.bfloat16 else 2.0 ** -10)     # <= 1 ulp at the top of [0, 6]
-    assert float((d > 0).float().mean()) < 0.02
-
-
-def test_expand_dw_rejects_unsupported_shapes():
-    from voice100_b200 import V100Error
-    x = K.empty_ncw(1, 64, 32, DEV)
-    W1 = torch.zeros(192, 64, device=DEV, dtype=torch.bfloat16)               # hidden width not a multiple of 256
-    z = torch.zeros(192, device=DEV)
-    with pytest.raises(V100Error):
-        K.expand_dw(x, W1, z, z, torch.zeros(192, 128, device=DEV, dtype=torch.int32), z, z, 11)
-    with pytest.raises(V100Error):
-        K.dw_pack_pairs(torch.zeros(8, 85, device=DEV, dtype=torch.bfloat16))  # k > 83
-
-
-# ------------------------------------------------------------------------------------------------
 # log-mel
 # ------------------------------------------------------------------------------------------------
 def test_logmel_matches_oracle_and_golden():

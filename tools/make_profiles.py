@@ -21,8 +21,6 @@ def short(name):
 
 
 def kind_of(name):
-    if "expand_dw" in name:
-        return "expand_dw"
     if "conv_gemm" in name:
         return "gemm"
     if "dw_" in name:

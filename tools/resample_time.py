@@ -8,8 +8,7 @@ Reports, with the card's name and power limit read in the same run:
       16 -> 48 kHz (fp32): CUDA events over `steps` calls after a warm-up.  Bytes are the input and output rows (the
       ~40 KB table is ignored); FLOPs are 2 x the packed taps of every output sample.  The bound is the larger of
       bytes / 7.7 TB/s and FLOPs / (148 SMs x 128 FMA/clk x 2 x the SM clock nvidia-smi reports right after the timed
-      loop); each row repeats with the packed table read through the read-only path instead of shared memory
-      (V100_RESAMPLE_TAPS=ldg, a child process).
+      loop).
   (t) torchaudio.functional.resample 44.1 -> 16 kHz on CUDA tensors of the same batch (CUDA events) and on the host
       with all threads (wall clock, a smaller batch), as input audio seconds per second.
   (g) the graphed v1 ASR step (asr_en_base, bench.py's model) on int16 PCM at 44.1 kHz against the same batch at 16 kHz.
@@ -121,20 +120,12 @@ def main():
     ap.add_argument("--steps", type=int, default=20)
     ap.add_argument("--host-batch", type=int, default=8)
     ap.add_argument("--out", default=os.path.join(ROOT, "profiles", "r05_resample.md"))
-    ap.add_argument("--kernels-json", action="store_true", help="print (k) as JSON and exit (used for the ldg child)")
     args = ap.parse_args()
     if not torch.cuda.is_available():
         sys.exit("resample_time.py needs a CUDA device")
-    if args.kernels_json:
-        print(json.dumps(kernel_rows(args.batch, args.seconds, args.steps)))
-        return
     card = subprocess.run(["nvidia-smi", "--id=0", "--query-gpu=name,power.limit", "--format=csv,noheader"],
                           stdout=subprocess.PIPE, text=True).stdout.strip()
     rows = kernel_rows(args.batch, args.seconds, args.steps)
-    child = subprocess.run([sys.executable, os.path.abspath(__file__), "--kernels-json", "--batch", str(args.batch),
-                            "--seconds", str(args.seconds), "--steps", str(args.steps)],
-                           env=dict(os.environ, V100_RESAMPLE_TAPS="ldg"), stdout=subprocess.PIPE, text=True, check=True)
-    ldg = json.loads(child.stdout.strip().splitlines()[-1])
     ta = torchaudio_rows(args.batch, args.seconds, args.steps, args.host_batch)
     asr = asr_rows(args.batch, args.seconds, args.steps)
 
@@ -144,14 +135,12 @@ def main():
              f"{args.steps} calls after a warm-up; the input is larger than L2 at every rate.", "",
              "## (k) the kernel alone", "",
              "Bytes: input + output rows.  FLOPs: 2 x packed taps per output.  Bound: the larger of bytes / 7.7 TB/s "
-             "and FLOPs / (148 x 128 FMA/clk x 2 x SM clock read by nvidia-smi right after the loop).  "
-             "`ldg`: the same kernel reading the packed table through the read-only path instead of shared memory.", "",
-             "| rate | input | ms | GB/s | TFLOP/s | SM MHz | bound by | share of bound | input audio-s/s | ldg ms |",
-             "|---|---|---|---|---|---|---|---|---|---|"]
-    for r, l in zip(rows, ldg):
+             "and FLOPs / (148 x 128 FMA/clk x 2 x SM clock read by nvidia-smi right after the loop).", "",
+             "| rate | input | ms | GB/s | TFLOP/s | SM MHz | bound by | share of bound | input audio-s/s |",
+             "|---|---|---|---|---|---|---|---|---|"]
+    for r in rows:
         lines.append(f"| {r['orig']} → {r['new']} | {r['input']} | {r['ms']:.3f} | {r['gbs']:.0f} | {r['tflops']:.2f} | "
-                     f"{r['sm_mhz']:.0f} | {r['bound_by']} | {r['share']:.2f} | {r['in_audio_s_per_s']:.3g} | "
-                     f"{l['ms']:.3f} |")
+                     f"{r['sm_mhz']:.0f} | {r['bound_by']} | {r['share']:.2f} | {r['in_audio_s_per_s']:.3g} |")
     lines += ["", "## (t) torchaudio.functional.resample, 44.1 → 16 kHz, fp32", "",
               f"- same GPU, CUDA tensors, {B} x {S} s: {ta['gpu_ms']:.2f} ms = {ta['gpu_audio_s_per_s']:.3g} input audio-s/s",
               f"- host, {ta['host_threads']} threads, {ta['host_batch']} x {S} s: {ta['host_s']:.2f} s = "
@@ -166,7 +155,7 @@ def main():
     print(text)
     with open(args.out, "w") as f:
         f.write(text)
-    print(json.dumps(dict(card=card, kernels=rows, ldg=ldg, torchaudio=ta, asr=asr)))
+    print(json.dumps(dict(card=card, kernels=rows, torchaudio=ta, asr=asr)))
 
 
 if __name__ == "__main__":

@@ -96,13 +96,6 @@ for dtype in (torch.bfloat16, torch.float16):
     for (Tb, kb) in ((1027, 35), (5, 19), (2049, 59)):
         xb = K.empty_ncw(3, 16, Tb, dev, dtype); xb.data.normal_()
         K.dwconv(xb, torch.randn(16, kb, device=dev).to(dtype), None, torch.zeros(16, device=dev), kb, 1, 1)
-    # the fused expand + depthwise kernel (opt-in path): ragged T, K not a multiple of 64, more units than CTA pairs
-    for (Bf, Ci, Hf, Tf, kf) in ((2, 72, 512, 333, 67), (3, 64, 256, 257, 11), (90, 64, 256, 70, 33)):
-        xf = K.empty_ncw(Bf, Ci, Tf, dev, dtype); xf.data.normal_()
-        W1 = torch.randn(Hf, Ci, device=dev).to(dtype)
-        wd = torch.randn(Hf, kf, device=dev).to(dtype)
-        z, o = torch.zeros(Hf, device=dev), torch.ones(Hf, device=dev)
-        K.expand_dw(xf, W1, o, z, K.dw_pack_pairs(wd), o, z, kf)
 lp = torch.log_softmax(torch.randn(3, 50, 29, device=dev), -1)
 v.ctc_best_path_batch(lp, torch.tensor([50, 30, 4]), torch.randint(1, 29, (3, 9), device=dev), torch.tensor([9, 5, 9]))
 torch.cuda.synchronize()

@@ -23,8 +23,6 @@ SIGNATURES = {
     "v100_conv1x1": [_p, _l, _p, _p, _p, _p, _p, _l, _i, _i, _i, _i, _i, _i, _p],
     "v100_conv1x1_f32out": [_p, _l, _p, _p, _p, _l, _i, _i, _i, _i, _i, _p],
     "v100_dwconv1d": [_p, _l, _p, _p, _p, _p, _l, _i, _i, _i, _i, _i, _i, _i, _p],
-    "v100_dw_pack_pairs": [_p, _p, _i, _i, _p],
-    "v100_expand_dw": [_p, _l, _p, _p, _p, _p, _p, _p, _p, _l, _i, _i, _i, _i, _i, _i, _p],
     "v100_dwconv1d_simt": [_p, _l, _p, _p, _p, _p, _l, _i, _i, _i, _i, _i, _i, _i, _p],
     "v100_convtranspose1d_k5s2": [_p, _l, _p, _p, _p, _p, _l, _i, _i, _i, _i, _i, _p],
     "v100_embedding_ncw16": [_p, _p, _p, _l, _i, _i, _i, _i, _p, _p],
@@ -50,7 +48,7 @@ SIGNATURES = {
     "v100_world_analyze": [_p, _i, _l, _p, _i, _l, _p, _p, _l, _p, _i, _p, _p, _p, _p, _p, _p],
 }
 
-ABI_VERSION = 8
+ABI_VERSION = 9
 _lib = None
 
 

@@ -8,8 +8,7 @@ bf16-packed copies built by `prepare_*` through the C ABI.
 """
 from __future__ import annotations
 
-import os
-from typing import List, Optional, Tuple
+from typing import Tuple
 
 import torch
 from torch import nn
@@ -50,33 +49,21 @@ class InvertedResidualParams(nn.Module):
         s1, b1 = fold_bn(e[1])
         s2, b2 = fold_bn(d[1])
         s3, b3 = fold_bn(bn3)
-        wd = d[0].weight.detach()[:, 0, :].to(dtype).contiguous()
-        # stride-1 blocks whose hidden width is a multiple of 256 run expand + depthwise as ONE kernel
-        fused = FUSE_EXPAND_DW and self.stride == 1 and self.hidden % 256 == 0 and self.c_in % 8 == 0 and \
-            self.kernel_size <= 83 and wd.is_cuda
         return dict(
             w1=e[0].weight.detach()[:, :, 0].to(dtype).contiguous(), s1=s1, b1=b1,
-            wd=wd, s2=s2, b2=b2, wd_pairs=K.dw_pack_pairs(wd) if fused else None,
+            wd=d[0].weight.detach()[:, 0, :].to(dtype).contiguous(), s2=s2, b2=b2,
             w2=p.weight.detach()[:, :, 0].to(dtype).contiguous(), s3=s3, b3=b3,
             k=self.kernel_size, stride=self.stride, res=self.use_residual)
 
 
-# V100_FUSE=1 in the environment runs expand + depthwise of the stride-1 blocks as ONE kernel (v100_expand_dw).  It is
-# correct (tests/test_kernels_gpu.py) but OFF by default: measured on the B200 it is slower than the two kernels it
-# replaces (DESIGN.md section 7 -- the depthwise FIR is bound by shared-memory wavefronts, not by HBM, so keeping the
-# 4x-wide tensor on chip buys nothing while the per-tile reload of the Toeplitz fragments costs a second FIR's worth).
-FUSE_EXPAND_DW = os.environ.get("V100_FUSE", "0") == "1"
+# Read by bench.py's per-kernel work model: expand and depthwise run as two kernels (DESIGN.md section 3.7).
+FUSE_EXPAND_DW = False
 
 
-def run_inverted_residual(x: K.Ncw, w: dict, fuse: Optional[bool] = None) -> K.Ncw:
-    """pw-expand (+BN+ReLU6) -> depthwise k (+BN+ReLU6) -> pw-project (+BN) (+x)   (asr.py:45-59).
-    Stride-1 blocks run the first two stages as the fused expand+depthwise kernel (the 4x-wide tensor between them
-    never touches HBM); `fuse=False` forces the three-kernel form."""
-    if w.get("wd_pairs") is not None and fuse is not False:
-        h = K.expand_dw(x, w["w1"], w["s1"], w["b1"], w["wd_pairs"], w["s2"], w["b2"], w["k"])
-    else:
-        h = K.conv1x1(x, w["w1"], w["s1"], w["b1"], K.ACT_RELU6)
-        h = K.dwconv(h, w["wd"], w["s2"], w["b2"], w["k"], w["stride"], K.ACT_RELU6)
+def run_inverted_residual(x: K.Ncw, w: dict) -> K.Ncw:
+    """pw-expand (+BN+ReLU6) -> depthwise k (+BN+ReLU6) -> pw-project (+BN) (+x)   (asr.py:45-59)."""
+    h = K.conv1x1(x, w["w1"], w["s1"], w["b1"], K.ACT_RELU6)
+    h = K.dwconv(h, w["wd"], w["s2"], w["b2"], w["k"], w["stride"], K.ACT_RELU6)
     return K.conv1x1(h, w["w2"], w["s3"], w["b3"], K.ACT_NONE, res=x if w["res"] else None)
 
 

@@ -1,7 +1,6 @@
 // extern "C" surface of libv100.so (see include/v100.h) + host plumbing.
 #include <cstdarg>
 #include <cstdio>
-#include <cstdlib>
 #include <mutex>
 
 #include "host.h"
@@ -16,14 +15,6 @@ int fail(int code, const char* fmt, ...) {
   vsnprintf(g_err, sizeof(g_err), fmt, ap);
   va_end(ap);
   return code;
-}
-
-bool pdl_enabled() {
-  static const bool on = [] {
-    const char* e = getenv("V100_PDL");
-    return e != nullptr && e[0] == '1';
-  }();
-  return on;
 }
 
 int num_sms() {
@@ -147,17 +138,6 @@ int v100_conv1x1_f32out(const void* x, int64_t x_pitch, const void* W, const flo
 int v100_dwconv1d(const void* x, int64_t x_pitch, const void* w, const float* scale, const float* shift, void* y,
                   int64_t y_pitch, int B, int C, int T_in, int k, int stride, int act, int dtype, void* stream) {
   return dwconv1d(x, x_pitch, w, scale, shift, y, y_pitch, B, C, T_in, k, stride, act, dtype, 0, STREAM(stream));
-}
-
-int v100_dw_pack_pairs(const void* w, uint32_t* pairs, int C, int k, void* stream) {
-  return dw_pack_pairs(w, pairs, C, k, STREAM(stream));
-}
-
-int v100_expand_dw(const void* x, int64_t x_pitch, const void* W1, const float* scale1, const float* shift1,
-                   const uint32_t* dw_pairs, const float* scale2, const float* shift2, void* y, int64_t y_pitch,
-                   int B, int C_in, int H, int T, int k, int dtype, void* stream) {
-  return expand_dw(x, x_pitch, W1, scale1, shift1, dw_pairs, scale2, shift2, y, y_pitch, B, C_in, H, T, k, dtype,
-                   STREAM(stream));
 }
 
 // Same contract as v100_dwconv1d but always the plain CUDA-core kernel (any stride); exported so the tests can

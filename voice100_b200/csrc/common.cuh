@@ -24,17 +24,6 @@ __device__ __forceinline__ bool elect_one() {
 }
 
 // ------------------------------------------------------------------------------------------
-// Programmatic dependent launch (host side: launch_pdl in host.h).  A kernel of the step calls pdl_trigger() as
-// soon as it starts -- once every CTA of the grid has done so (i.e. the last wave is resident) the NEXT kernel of the
-// stream may be launched into whatever SM resources free up, so its launch latency and prologue (barrier init, TMEM
-// allocation, tensor-map prefetch, filter staging) overlap this kernel's tail -- and pdl_wait() before its first
-// access to global memory another kernel of the chain produces or still reads: the wait returns only when the
-// preceding kernel has completed and its writes are visible.  Both are no-ops for a launch without the attribute.
-// ------------------------------------------------------------------------------------------
-__device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
-__device__ __forceinline__ void pdl_trigger() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
-
-// ------------------------------------------------------------------------------------------
 // mbarrier
 // ------------------------------------------------------------------------------------------
 __device__ __forceinline__ void mbar_init(uint64_t* bar, uint32_t count) {

@@ -37,8 +37,6 @@
 #include "common.cuh"
 #include "host.h"
 
-#include <cstdlib>
-
 namespace v100 {
 
 constexpr int kBlockM = 128;
@@ -138,7 +136,6 @@ __device__ __forceinline__ void conv_gemm_body(const CUtensorMap& tm_w, const CU
   const int warp = __shfl_sync(0xffffffffu, threadIdx.x >> 5, 0);  // provably warp-uniform for the compiler
   const int lane = threadIdx.x & 31;
 
-  pdl_trigger();   // persistent grid: every CTA is resident, the next kernel may queue up behind our tail
   if (warp == 0 && lane == 0) {
     if (!WRES) tma_prefetch_desc(&tm_w);
     tma_prefetch_desc(&tm_x);
@@ -174,10 +171,9 @@ __device__ __forceinline__ void conv_gemm_body(const CUtensorMap& tm_w, const CU
   const uint32_t tmem_base = *tmem_slot;
 
   if constexpr (WRES) {
-    // This CTA's 128 weight rows -> tensor memory, straight from global memory (weights are not produced by the
-    // preceding kernel, so this runs in front of pdl_wait): TMEM lane = output channel, and a row-major 16-bit row
-    // already is "two K elements per 32-bit column".  The two epilogue warps of a lane quadrant alternate
-    // 32-column blocks.
+    // This CTA's 128 weight rows -> tensor memory, straight from global memory: TMEM lane = output channel, and a
+    // row-major 16-bit row already is "two K elements per 32-bit column".  The two epilogue warps of a lane quadrant
+    // alternate 32-column blocks.
     if (warp >= 4) {
       const int q = warp & 3, g = (warp - 4) >> 2;
       const int ch = ((tile0 % p.m_tiles) * CG + int(cta_rank)) * kBlockM + q * 32 + lane;
@@ -197,7 +193,6 @@ __device__ __forceinline__ void conv_gemm_body(const CUtensorMap& tm_w, const CU
     cluster_sync_all();   // the leader's MMAs read both CTAs' halves
     tc_fence_after();
   }
-  pdl_wait();      // everything above overlapped the previous kernel's tail; from here on we read its output
 
   if (warp == 0) {
     // ===================== TMA producer =====================
@@ -576,7 +571,8 @@ static int launch_gemm_e(const CUtensorMap& tw, const CUtensorMap& tx, const CUt
     configured_dev = dev;
   }
   const int grid = p.num_tiles < num_sms() ? p.num_tiles : num_sms();
-  V100_CUDA(launch_pdl(kern, dim3(grid), dim3(kGemmThreads), Cfg::kSmemBytes, stream, tw, tx, ty, tr, p));
+  kern<<<dim3(grid), dim3(kGemmThreads), Cfg::kSmemBytes, stream>>>(tw, tx, ty, tr, p);
+  V100_CUDA(cudaGetLastError());
   return 0;
 }
 
@@ -625,10 +621,9 @@ static int launch_gemm_pair_e(const CUtensorMap& tw, const CUtensorMap& tx, cons
     configured_dev = dev;
   }
   int pairs = num_sms() / 2;
-  static const int cap = getenv("V100_GEMM_PAIRS") ? atoi(getenv("V100_GEMM_PAIRS")) : 0;   // experiments: fewer SMs
-  if (cap > 0 && cap < pairs) pairs = cap;
   if (p.num_tiles < pairs) pairs = p.num_tiles;
-  V100_CUDA(launch_pdl(kern, dim3(2 * pairs), dim3(kGemmThreads), Cfg::kSmemBytes, stream, tw, tx, ty, tr, p));
+  kern<<<dim3(2 * pairs), dim3(kGemmThreads), Cfg::kSmemBytes, stream>>>(tw, tx, ty, tr, p);
+  V100_CUDA(cudaGetLastError());
   return 0;
 }
 
@@ -658,7 +653,8 @@ static int launch_gemm_wres_e(const CUtensorMap& tx, const CUtensorMap& ty, cons
     V100_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::kSmemBytes));
     configured_dev = dev;
   }
-  V100_CUDA(launch_pdl(kern, dim3(2 * pairs), dim3(kGemmThreads), Cfg::kSmemBytes, stream, tx, ty, tr, p));
+  kern<<<dim3(2 * pairs), dim3(kGemmThreads), Cfg::kSmemBytes, stream>>>(tx, ty, tr, p);
+  V100_CUDA(cudaGetLastError());
   return 0;
 }
 
@@ -672,8 +668,7 @@ static int launch_gemm_wres(const CUtensorMap& tx, const CUtensorMap& ty, const 
 // WRES applies when the pair's weight block fits in tensor memory next to two 128-column accumulators and the
 // channel blocks divide the device's pairs without leaving more than ~5 % of them idle.
 static int wres_pairs(int C_in, int C_out, int B, int T) {
-  static const int enabled = getenv("V100_GEMM_WRES") ? atoi(getenv("V100_GEMM_WRES")) : 1;  // A/B runs
-  if (!enabled || C_in > 512 || C_in % 128 != 0 || C_out % (2 * kBlockM) != 0) return 0;
+  if (C_in > 512 || C_in % 128 != 0 || C_out % (2 * kBlockM) != 0) return 0;
   const int m_tiles = C_out / (2 * kBlockM), all = num_sms() / 2;
   const int slots = all / m_tiles;
   if (slots < 1 || slots * m_tiles * 20 < all * 19) return 0;
@@ -725,8 +720,7 @@ int conv1x1(const void* x, int64_t x_pitch, const void* W, const float* scale, c
   p.n_taps = 1; p.tap_xrow[0] = 0; p.tap_acc[0] = 0;
   p.scale = scale; p.shift = shift; p.act = act; p.has_res = res != nullptr; p.dtype = dtype;
   p.t_tiles = (T + bn - 1) / bn;
-  static const int force_cg = getenv("V100_GEMM_CG") ? atoi(getenv("V100_GEMM_CG")) : 0;  // debugging / A-B runs
-  if (const int pairs = force_cg != 1 ? wres_pairs(C_in, C_out, B, T) : 0) {
+  if (const int pairs = wres_pairs(C_in, C_out, B, T)) {
     CUtensorMap txw;   // [64 steps x 128 k rows] boxes: one per ring stage and CTA
     if (int e = make_tmap_3d(&txw, tmap_type(dtype), x, T, C_in, B, x_pitch * 2, int64_t(C_in) * x_pitch * 2, 64, 128)) return e;
     p.w_raw = static_cast<const unsigned short*>(W);
@@ -736,7 +730,7 @@ int conv1x1(const void* x, int64_t x_pitch, const void* W, const float* scale, c
     p.num_tiles = p.m_tiles * p.t_tiles * B;
     return launch_gemm_wres(txw, ty, tr, p, pairs, stream);
   }
-  if (C_out % (2 * kBlockM) == 0 && force_cg != 1) {   // CTA pairs; 128-column tiles where they pad the row less
+  if (C_out % (2 * kBlockM) == 0) {   // CTA pairs; 128-column tiles where they pad the row less
     p.m_tiles = C_out / (2 * kBlockM);
     p.num_tiles = p.m_tiles * p.t_tiles * B;
     return launch_gemm_pair(tw, tx, ty, tr, p, bn, stream);

@@ -98,7 +98,6 @@ dw_tc_kernel(const __grid_constant__ CUtensorMap tm_x, const unsigned short* __r
   const int n_box = 2 * (n_t - 1) + NCH;           // boxes per work unit
   constexpr uint32_t kAcc0 = 0, kA0 = 256;         // TMEM columns: accumulators 0 / 128, Toeplitz buffers 256 / 384
 
-  pdl_trigger();
   if (warp == 0 && lane == 0) {
     tma_prefetch_desc(&tm_x);
   }
@@ -122,7 +121,6 @@ dw_tc_kernel(const __grid_constant__ CUtensorMap tm_x, const unsigned short* __r
   __syncthreads();
   tc_fence_after();
   const uint32_t tmem_base = *tmem_slot;
-  pdl_wait();      // (x is the previous kernel's output)
 
   if (warp == 0) {
     // ===================== TMA producer =====================
@@ -341,7 +339,6 @@ dw_bulk_kernel(const unsigned short* __restrict__ x, long long x_pitch, const un
   const int cs = max(tcA, 0), ce = max(min(tcA + need, T8), cs);
   const uint32_t bytes = uint32_t(ce - cs) * 2u;
   const int dst_off = cs - tcA;
-  pdl_trigger();
 
   // zero both buffers once (halo left of the clip, everything right of the copied span), barriers
   for (int i = lane; i < 2 * kDwRow / 8; i += 32)
@@ -353,7 +350,6 @@ dw_bulk_kernel(const unsigned short* __restrict__ x, long long x_pitch, const un
   }
   fence_proxy_async();     // the zeros (generic proxy) are ordered before the bulk copies (async proxy) into the same rows
   __syncwarp();
-  pdl_wait();              // (x is the previous kernel's output)
   // the clip's last T & 7 samples (staged index tail0 + lane), when the tiles read them
   const int tail0 = T8 - tcA;
   const bool has_tail = lane < (T & 7) && tail0 >= 0 && tail0 + lane < need;
@@ -493,7 +489,6 @@ dw_s2_mma_kernel(const unsigned short* __restrict__ x, long long x_pitch, const 
   const int P2 = (D + 7) & ~7;                    // the staged phase arrays start at x_e / x_o index oc0 - P2
   const int s = P2 - D;                           // tiles start s outputs before oc0 (even)
   const int iA = oc0 - P2;                        // phase index of staged sample 0 (x index 2 iA, a multiple of 16)
-  pdl_trigger();
   if (c >= C) return;
 
   const int len = min(kDwChunk, T_out - oc0);
@@ -530,7 +525,6 @@ dw_s2_mma_kernel(const unsigned short* __restrict__ x, long long x_pitch, const 
   const bool relu6 = act == V100_ACT_RELU6;
   unsigned short* xs_e = xs_all[warp][0];
   unsigned short* xs_o = xs_all[warp][1];
-  pdl_wait();
 
   // The row passes through registers on its way to shared memory (cp.async cannot split 16-bit samples by parity), so
   // the NEXT row's 16-byte loads are issued before this row's MMAs and are in flight while they run: with the loads
@@ -630,7 +624,6 @@ dw_s2_kernel(const unsigned short* __restrict__ x, long long x_pitch, const unsi
   __shared__ __align__(8) float ws_all[kDwWarps][2 * kS2MaxWords];
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int c = blockIdx.y * kDwWarps + warp;
-  pdl_trigger();
   if (c >= C) return;
   const int b = blockIdx.z;
   const int oc0 = blockIdx.x * kS2Chunk;
@@ -639,7 +632,6 @@ dw_s2_kernel(const unsigned short* __restrict__ x, long long x_pitch, const unsi
   const int e = p8 - p;                       // xs[2*ol + j + e] = x[2*(oc0+ol) + j - p]
   unsigned short* xs = xs_all[warp];
   float* ws = ws_all[warp];
-  pdl_wait();
   const unsigned short* xrow = x + (static_cast<long long>(b) * C + c) * x_pitch;
   const int ia = 2 * oc0 - p8;
   for (int v = lane; v < kS2Row / 8; v += 32) {
@@ -694,8 +686,6 @@ dw_simt_kernel(const unsigned short* __restrict__ x, long long x_pitch, const un
                long long y_pitch, int C, int T_in, int T_out, int k, int stride, int act) {
   const int c = blockIdx.y, b = blockIdx.z;
   const int o0 = (blockIdx.x * 128 + threadIdx.x) * 8;
-  pdl_trigger();
-  pdl_wait();
   if (o0 >= T_out) return;
   const int p = (k - 1) >> 1;
   const unsigned short* xrow = x + (static_cast<long long>(b) * C + c) * x_pitch;
@@ -729,7 +719,8 @@ static int launch_dw_tc_k(const CUtensorMap& tx, const unsigned short* w, const 
   auto kern = dw_tc_kernel<NP, RELU6, DT>;
   V100_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, kTcSmem));
   const int grid = C < num_sms() ? C : num_sms();
-  V100_CUDA(launch_pdl(kern, dim3(grid), dim3(384), kTcSmem, stream, tx, w, scale, shift, y, y_pitch, B, C, T, k, N));
+  kern<<<dim3(grid), dim3(384), kTcSmem, stream>>>(tx, w, scale, shift, y, y_pitch, B, C, T, k, N);
+  V100_CUDA(cudaGetLastError());
   return 0;
 }
 
@@ -770,7 +761,7 @@ int dwconv1d(const void* x, int64_t x_pitch, const void* w, const float* scale, 
     dim3 grid((T_in + kDwChunk - 1) / kDwChunk, C / kDwWarps, (B + kDwRowsPerWarp - 1) / kDwRowsPerWarp);
     const long long xpl = x_pitch, ypl = y_pitch;
 #define V100_BULK(QQ, RL, DTT) \
-    launch_pdl(dw_bulk_kernel<QQ, RL, DTT>, grid, dim3(kDwWarps * 32), 0, stream, xp, xpl, wp, scale, shift, yp, ypl, B, C, T_in, k)
+    dw_bulk_kernel<QQ, RL, DTT><<<grid, dim3(kDwWarps * 32), 0, stream>>>(xp, xpl, wp, scale, shift, yp, ypl, B, C, T_in, k)
 #define V100_BULK_Q(QQ)                                                                                                   \
     do {                                                                                                                  \
       if (dtype == DT_F16) { if (act == V100_ACT_RELU6) V100_BULK(QQ, true, DT_F16); else V100_BULK(QQ, false, DT_F16); } \
@@ -807,9 +798,9 @@ int dwconv1d(const void* x, int64_t x_pitch, const void* w, const float* scale, 
 #define V100_S2(QQ, NV)                                                                                                     \
     do {                                                                                                                    \
       if (dtype == DT_F16)                                                                                                  \
-        launch_pdl(dw_s2_mma_kernel<QQ, DT_F16, NV>, grid, dim3(kDwWarps * 32), 0, stream, xp, xpl, wp, scale, shift, yp, ypl, B, C, T_in, T_out, k, act); \
+        dw_s2_mma_kernel<QQ, DT_F16, NV><<<grid, dim3(kDwWarps * 32), 0, stream>>>(xp, xpl, wp, scale, shift, yp, ypl, B, C, T_in, T_out, k, act); \
       else                                                                                                                  \
-        launch_pdl(dw_s2_mma_kernel<QQ, DT_BF16, NV>, grid, dim3(kDwWarps * 32), 0, stream, xp, xpl, wp, scale, shift, yp, ypl, B, C, T_in, T_out, k, act); \
+        dw_s2_mma_kernel<QQ, DT_BF16, NV><<<grid, dim3(kDwWarps * 32), 0, stream>>>(xp, xpl, wp, scale, shift, yp, ypl, B, C, T_in, T_out, k, act); \
     } while (0)
     if (Qs <= 2) { if (small) V100_S2(2, 7); else V100_S2(2, 11); }
     else { if (small) V100_S2(3, 7); else V100_S2(3, 11); }
@@ -818,16 +809,16 @@ int dwconv1d(const void* x, int64_t x_pitch, const void* w, const float* scale, 
     dim3 grid((T_out + kS2Chunk - 1) / kS2Chunk, (C + kDwWarps - 1) / kDwWarps, B);
     const long long xpl = x_pitch, ypl = y_pitch;
     if (dtype == DT_F16)
-      launch_pdl(dw_s2_kernel<DT_F16>, grid, dim3(kDwWarps * 32), 0, stream, xp, xpl, wp, scale, shift, yp, ypl, C, T_in, T_out, k, act);
+      dw_s2_kernel<DT_F16><<<grid, dim3(kDwWarps * 32), 0, stream>>>(xp, xpl, wp, scale, shift, yp, ypl, C, T_in, T_out, k, act);
     else
-      launch_pdl(dw_s2_kernel<DT_BF16>, grid, dim3(kDwWarps * 32), 0, stream, xp, xpl, wp, scale, shift, yp, ypl, C, T_in, T_out, k, act);
+      dw_s2_kernel<DT_BF16><<<grid, dim3(kDwWarps * 32), 0, stream>>>(xp, xpl, wp, scale, shift, yp, ypl, C, T_in, T_out, k, act);
   } else {
     dim3 grid((T_out + 1023) / 1024, C, B);
     const long long xpl = x_pitch, ypl = y_pitch;
     if (dtype == DT_F16)
-      launch_pdl(dw_simt_kernel<DT_F16>, grid, dim3(128), 0, stream, xp, xpl, wp, scale, shift, yp, ypl, C, T_in, T_out, k, stride, act);
+      dw_simt_kernel<DT_F16><<<grid, dim3(128), 0, stream>>>(xp, xpl, wp, scale, shift, yp, ypl, C, T_in, T_out, k, stride, act);
     else
-      launch_pdl(dw_simt_kernel<DT_BF16>, grid, dim3(128), 0, stream, xp, xpl, wp, scale, shift, yp, ypl, C, T_in, T_out, k, stride, act);
+      dw_simt_kernel<DT_BF16><<<grid, dim3(128), 0, stream>>>(xp, xpl, wp, scale, shift, yp, ypl, C, T_in, T_out, k, stride, act);
   }
   V100_CUDA(cudaGetLastError());
   return 0;

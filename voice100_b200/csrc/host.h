@@ -21,28 +21,6 @@ int num_sms();
       return ::v100::fail(static_cast<int>(e__), "%s -> %s", #expr, cudaGetErrorString(e__)); \
   } while (0)
 
-// Launch with programmatic stream serialization (see pdl_wait / pdl_trigger in common.cuh): the kernel may start
-// while the previous kernel of the stream is still draining.  ONLY for kernels that call pdl_wait() before touching
-// data of the chain.  Opt-in: V100_PDL=1 in the environment sets the attribute; the default is plain stream order,
-// because three alternating same-box A/B runs of the 30-kernel step showed no gain (6.59-6.77 ms with, 6.62-6.64 ms
-// without: the CUDA-graph step already equals the sum of its kernels, profiles/r02_history.md).
-bool pdl_enabled();
-template <typename... KArgs, typename... Args>
-inline cudaError_t launch_pdl(void (*kern)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t stream,
-                              Args&&... args) {
-  cudaLaunchConfig_t cfg{};
-  cfg.gridDim = grid;
-  cfg.blockDim = block;
-  cfg.dynamicSmemBytes = smem;
-  cfg.stream = stream;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  attr[0].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = attr;
-  cfg.numAttrs = pdl_enabled() ? 1 : 0;
-  return cudaLaunchKernelEx(&cfg, kern, static_cast<KArgs>(args)...);
-}
-
 // 16-bit tensor maps, 128-byte swizzle, zero fill out of bounds.  Dimensions innermost first.
 int make_tmap_2d(CUtensorMap* m, CUtensorMapDataType type, const void* base, int64_t d0, int64_t d1, int64_t stride1_bytes, int box0, int box1);
 int make_tmap_3d(CUtensorMap* m, CUtensorMapDataType type, const void* base, int64_t d0, int64_t d1, int64_t d2, int64_t stride1_bytes,
@@ -57,10 +35,6 @@ int conv1x1_f32out(const void* x, int64_t x_pitch, const void* W, const float* b
                    int B, int C_in, int C_out, int T, int dtype, cudaStream_t stream);
 int convtranspose1d_k5s2(const void* x, int64_t x_pitch, const void* Wp, const float* bias, void* workspace, void* y,
                          int64_t y_pitch, int B, int C_in, int C_out, int T, int dtype, cudaStream_t stream);
-int dw_pack_pairs(const void* w, uint32_t* pairs, int C, int k, cudaStream_t stream);
-int expand_dw(const void* x, int64_t x_pitch, const void* W1, const float* scale1, const float* shift1,
-              const uint32_t* dw_pairs, const float* scale2, const float* shift2, void* y, int64_t y_pitch, int B,
-              int C_in, int H, int T, int k, int dtype, cudaStream_t stream);
 int dwconv1d(const void* x, int64_t x_pitch, const void* w, const float* scale, const float* shift, void* y,
              int64_t y_pitch, int B, int C, int T_in, int k, int stride, int act, int dtype, int force_simt,
              cudaStream_t stream);

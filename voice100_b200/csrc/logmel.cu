@@ -24,8 +24,6 @@
 #include "host.h"
 #include "logmel_core.h"
 
-#include <cstdlib>
-
 namespace v100 {
 
 constexpr int kNMels = 64;
@@ -33,10 +31,11 @@ constexpr int kNFft = 512, kWin = 400, kHop = 160, kWinLeft = (kNFft - kWin) / 2
 constexpr int kMelTile = 32;         // frames per tile
 constexpr int kPStride = 33;
 constexpr int kMelMaxNnz = 1024;     // accepted filter-bank size (the HTK bank at 512/16 kHz/64 has 500 weights)
+constexpr int kMelWarps = 16;        // warps per CTA
+constexpr int kMelCtasPerSm = 2;     // resident CTAs per SM: the launch bounds and the persistent grid
 
-template <int NW>
 struct MelCfg {
-  static constexpr int kHalfWarps = 2 * NW;
+  static constexpr int kHalfWarps = 2 * kMelWarps;
   static constexpr int kIters = kMelTile / kHalfWarps;          // FFT passes per tile
   static constexpr int kWinBytes = 256 * 8;                     // float2 window of samples (2n, 2n+1)
   static constexpr int kTwBytes = 16 * 16 * 8;                  // W256^(q k1) as [k1][q]
@@ -65,24 +64,22 @@ struct MelParams {
   int tiles_per_clip, total_tiles;
 };
 
-template <int NW, bool I16>
-__global__ void __launch_bounds__(NW * 32, NW == 16 ? 2 : 3)
+template <bool I16>
+__global__ void __launch_bounds__(kMelWarps * 32, kMelCtasPerSm)
 logmel_kernel(const MelParams p) {
-  using Cfg = MelCfg<NW>;
   extern __shared__ __align__(16) uint8_t mel_smem[];
-  float2* win2 = reinterpret_cast<float2*>(mel_smem);                                   // [256]
-  cpx* twt = reinterpret_cast<cpx*>(mel_smem + Cfg::kWinBytes);                         // [16 k1][16 q]
-  int* fbs = reinterpret_cast<int*>(mel_smem + Cfg::kWinBytes + Cfg::kTwBytes);         // [3][64]
-  cpx* exch = reinterpret_cast<cpx*>(mel_smem + Cfg::kWinBytes + Cfg::kTwBytes + Cfg::kFbBytes);
-  float* P = reinterpret_cast<float*>(reinterpret_cast<uint8_t*>(exch) + Cfg::kEBytes);  // [257][33]
-  float* otile = reinterpret_cast<float*>(exch);                                        // [32][65] (NTC mode)
+  float2* win2 = reinterpret_cast<float2*>(mel_smem);                                      // [256]
+  cpx* twt = reinterpret_cast<cpx*>(mel_smem + MelCfg::kWinBytes);                          // [16 k1][16 q]
+  int* fbs = reinterpret_cast<int*>(mel_smem + MelCfg::kWinBytes + MelCfg::kTwBytes);       // [3][64]
+  cpx* exch = reinterpret_cast<cpx*>(mel_smem + MelCfg::kWinBytes + MelCfg::kTwBytes + MelCfg::kFbBytes);
+  float* P = reinterpret_cast<float*>(reinterpret_cast<uint8_t*>(exch) + MelCfg::kEBytes);  // [257][33]
+  float* otile = reinterpret_cast<float*>(exch);                                           // [32][65] (NTC mode)
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const float in_scale = I16 ? (1.0f / 32768.0f) : 1.0f;
-  pdl_trigger();
 
   // ---- once per CTA: window, twiddles, filter descriptors ----
-  for (int n = threadIdx.x; n < 256; n += NW * 32) {   // periodic Hann(400) centred in the 512 frame
+  for (int n = threadIdx.x; n < 256; n += kMelWarps * 32) {   // periodic Hann(400) centred in the 512 frame
     float w2[2];
 #pragma unroll
     for (int h = 0; h < 2; ++h) {
@@ -91,7 +88,7 @@ logmel_kernel(const MelParams p) {
     }
     win2[n] = make_float2(w2[0], w2[1]);
   }
-  for (int i = threadIdx.x; i < 256; i += NW * 32) {   // twt[k1][q] = exp(-2 pi i q k1 / 256)
+  for (int i = threadIdx.x; i < 256; i += kMelWarps * 32) {   // twt[k1][q] = exp(-2 pi i q k1 / 256)
     const int k1 = i >> 4, qq = i & 15;
     float sn, cs;
     sincospif(-float((2 * qq * k1) & 511) / 256.0f, &sn, &cs);
@@ -129,7 +126,6 @@ logmel_kernel(const MelParams p) {
   const int partner_lane = (lane & 16) | ((16 - q) & 15);
   const float blank = p.out_mode == V100_MEL_POWER_F32_NCW ? 0.0f : logf(p.log_offset);
   __syncthreads();
-  pdl_wait();   // the tables above overlapped the previous kernel; the waveform / output buffers may still be in use by it
 
   for (int tile = blockIdx.x; tile < p.total_tiles; tile += gridDim.x) {
     const int b = tile / p.tiles_per_clip;
@@ -143,8 +139,8 @@ logmel_kernel(const MelParams p) {
 
     // ---------------- FFT phase: one frame per half-warp and pass ----------------
 #pragma unroll 1
-    for (int it = 0; it < Cfg::kIters; ++it) {
-      const int fl = warp + NW * it + 16 * half;       // the two frames of a warp are 16 apart (P bank layout)
+    for (int it = 0; it < MelCfg::kIters; ++it) {
+      const int fl = warp + kMelWarps * it + 16 * half;   // the two frames of a warp are 16 apart (P bank layout)
       const int t = f0 + fl;
       const bool valid = t < n_frames;
       if (!__any_sync(0xffffffffu, valid)) continue;   // nothing to transform; the mel phase writes `blank`
@@ -225,7 +221,7 @@ logmel_kernel(const MelParams p) {
       const bool valid = t < n_frames;
       const float* Pl = P + lane;
 #pragma unroll 1
-      for (int m = warp; m < kNMels; m += NW) {
+      for (int m = warp; m < kNMels; m += kMelWarps) {
         const int s0 = fbs[m], cnt4 = fbs[kNMels + m];            // taps, rounded up to four (zero weights)
         const float4* w4 = reinterpret_cast<const float4*>(fbw + fbs[2 * kNMels + m]);
         // (a padded tap may point one to three rows past the filter: clamp the row, its weight is zero)
@@ -256,7 +252,7 @@ logmel_kernel(const MelParams p) {
     }
     __syncthreads();
     if (p.out_mode == V100_MEL_LOG_F32_NTC) {   // out[b][t][64]: transpose through the tile
-      for (int i = threadIdx.x; i < kMelTile * (kNMels / 4); i += NW * 32) {
+      for (int i = threadIdx.x; i < kMelTile * (kNMels / 4); i += kMelWarps * 32) {
         const int fl = i >> 4, m4 = (i & 15) * 4;
         const int t = f0 + fl;
         if (t < p.T) {
@@ -270,20 +266,19 @@ logmel_kernel(const MelParams p) {
   }
 }
 
-template <int NW, bool I16>
+template <bool I16>
 static int launch_logmel(const MelParams& p, cudaStream_t stream) {
-  using Cfg = MelCfg<NW>;
-  auto kern = logmel_kernel<NW, I16>;
+  auto kern = logmel_kernel<I16>;
   static thread_local int configured_dev = -1;
   int dev = 0;
   V100_CUDA(cudaGetDevice(&dev));
   if (configured_dev != dev) {
-    V100_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::kSmemBytes));
+    V100_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, MelCfg::kSmemBytes));
     configured_dev = dev;
   }
-  const int per_sm = NW == 16 ? 2 : 3;
-  const int grid = p.total_tiles < per_sm * num_sms() ? p.total_tiles : per_sm * num_sms();
-  V100_CUDA(launch_pdl(kern, dim3(grid), dim3(NW * 32), Cfg::kSmemBytes, stream, p));
+  const int grid = p.total_tiles < kMelCtasPerSm * num_sms() ? p.total_tiles : kMelCtasPerSm * num_sms();
+  kern<<<dim3(grid), dim3(kMelWarps * 32), MelCfg::kSmemBytes, stream>>>(p);
+  V100_CUDA(cudaGetLastError());
   return 0;
 }
 
@@ -319,9 +314,7 @@ int logmel(const void* wav, int wav_dtype, const int32_t* len, int B, int64_t wa
   const long long total = static_cast<long long>(p.tiles_per_clip) * B;
   if (total > 2147483647LL) return fail(V100_E_UNSUPPORTED, "logmel: too many tiles");
   p.total_tiles = int(total);
-  static const int nw = getenv("V100_MEL_WARPS") ? atoi(getenv("V100_MEL_WARPS")) : 16;   // A/B runs
-  if (nw == 8) return wav_dtype == V100_WAV_I16 ? launch_logmel<8, true>(p, stream) : launch_logmel<8, false>(p, stream);
-  return wav_dtype == V100_WAV_I16 ? launch_logmel<16, true>(p, stream) : launch_logmel<16, false>(p, stream);
+  return wav_dtype == V100_WAV_I16 ? launch_logmel<true>(p, stream) : launch_logmel<false>(p, stream);
 }
 
 // ------------------------------------------------------------------------------------------------------------------

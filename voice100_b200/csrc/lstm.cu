@@ -9,8 +9,6 @@
 #include "common.cuh"
 #include "host.h"
 
-#include <cstdlib>
-
 namespace v100 {
 
 // ------------------------------------------------------------------------------------------------
@@ -330,19 +328,17 @@ static int lstm_layer_pair(const void* gx, const void* w_hh, const int32_t* leng
   cfg.blockDim = dim3(kPairThreads);
   cfg.dynamicSmemBytes = smem;
   cfg.stream = stream;
-  cudaLaunchAttribute attrs[1];                 // (the cluster shape is the kernel's compile-time __cluster_dims__)
-  attrs[0].id = cudaLaunchAttributeCooperative;
-  attrs[0].val.cooperative = 1;
-  cfg.attrs = attrs;
-  cfg.numAttrs = 0;
   cfg.gridDim = dim3(2 * p.pairs * 2);          // one group: 2 directions x pairs clusters x 2 CTAs
   int max_clusters = 0;
   V100_CUDA(cudaOccupancyMaxActiveClusters(&max_clusters, kern, &cfg));
   const int max_groups = max_clusters / (2 * p.pairs);
   if (max_groups < 1)
     return fail(V100_E_UNSUPPORTED, "lstm_layer: H=%d needs %d co-resident CTA pairs, this device fits %d", H, 2 * p.pairs, max_clusters);
-  static const bool cooperative = getenv("V100_LSTM_NONCOOP") == nullptr;
-  cfg.numAttrs = cooperative ? 1 : 0;
+  cudaLaunchAttribute attrs[1];                 // (the cluster shape is the kernel's compile-time __cluster_dims__)
+  attrs[0].id = cudaLaunchAttributeCooperative;
+  attrs[0].val.cooperative = 1;
+  cfg.attrs = attrs;
+  cfg.numAttrs = 1;
   for (int g0 = 0; g0 < p.groups_total; g0 += max_groups) {
     p.group0 = g0;
     p.groups = p.groups_total - g0 < max_groups ? p.groups_total - g0 : max_groups;

@@ -185,8 +185,6 @@ ctc_finalize_kernel(const float* __restrict__ y, long long pitch, float* __restr
                     int32_t* __restrict__ out_len) {
   const int b = blockIdx.y;
   const int t = blockIdx.x * 128 + threadIdx.x;
-  pdl_trigger();
-  pdl_wait();
   // ConvVoiceEncoder.output_length (asr.py:81-82): (audio_len + 1) // 2, emitted here so the pipeline needs no
   // separate element-wise launch
   if (out_len != nullptr && blockIdx.x == 0 && threadIdx.x == 0) out_len[b] = (audio_len[b] + 1) / 2;
@@ -210,8 +208,9 @@ int ctc_finalize(const float* y_ncw, int64_t y_pitch, float* logits, int64_t* to
   if ((audio_len == nullptr) != (out_len == nullptr)) return fail(V100_E_INVALID, "ctc_finalize: audio_len and out_len go together");
   if (B <= 0 || V <= 0 || T <= 0 || B > 65535 || y_pitch < T) return fail(V100_E_INVALID, "ctc_finalize: bad sizes");
   dim3 grid((T + 127) / 128, B);
-  V100_CUDA(launch_pdl(ctc_finalize_kernel, grid, dim3(128), 0, stream, y_ncw, static_cast<long long>(y_pitch), logits,
-                       tokens, V, T, audio_len, out_len));
+  ctc_finalize_kernel<<<grid, dim3(128), 0, stream>>>(y_ncw, static_cast<long long>(y_pitch), logits, tokens, V, T,
+                                                      audio_len, out_len);
+  V100_CUDA(cudaGetLastError());
   return 0;
 }
 
@@ -418,8 +417,6 @@ int ncw_f32_to_ntc(const float* y_ncw, int64_t y_pitch, float* out, int B, int C
 __global__ void __launch_bounds__(256)
 maskaudio_kernel(const float* __restrict__ audio, const int32_t* __restrict__ audio_len, float* __restrict__ out,
                  long long n, int T, int C, float log_offset) {
-  pdl_trigger();
-  pdl_wait();
   const long long tc = static_cast<long long>(T) * C;
   for (long long i = blockIdx.x * 256LL + threadIdx.x; i < n; i += gridDim.x * 256LL) {
     const long long b = i / tc;
@@ -438,8 +435,8 @@ int maskaudio(const float* audio, const int32_t* audio_len, float* out, int B, i
   long long blocks = (n + 255) / 256;
   const long long cap = 32LL * num_sms();
   if (blocks > cap) blocks = cap;
-  V100_CUDA(launch_pdl(maskaudio_kernel, dim3((unsigned)blocks), dim3(256), 0, stream, audio, audio_len, out, n, T, C,
-                       log_offset));
+  maskaudio_kernel<<<dim3((unsigned)blocks), dim3(256), 0, stream>>>(audio, audio_len, out, n, T, C, log_offset);
+  V100_CUDA(cudaGetLastError());
   return 0;
 }
 

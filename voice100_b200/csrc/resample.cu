@@ -14,8 +14,6 @@
 //    write consecutive samples); each output is its own fixed-order fmaf chain over the phase's taps, so results are
 //    bit-identical from run to run and do not depend on the rest of the batch.  One tap load serves R outputs.
 //  - all sample indices are int64 (j o overflows int32 at 15 s x 441).
-#include <stdlib.h>
-
 #include "common.cuh"
 #include "host.h"
 
@@ -53,8 +51,6 @@ resample_kernel(const void* __restrict__ x, long long x_pitch, const int32_t* __
   const int span = (JT - 1) * o + K;
   float* xs = smem;
   const float* tp = taps;
-  pdl_trigger();
-  pdl_wait();
   const int b = blockIdx.y;
   int lb = __ldg(len + b);
   lb = lb < 0 ? 0 : (lb > L_in ? L_in : lb);
@@ -117,16 +113,6 @@ resample_kernel(const void* __restrict__ x, long long x_pitch, const int32_t* __
   }
 }
 
-// measurement switch: V100_RESAMPLE_TAPS=ldg reads the packed table through the read-only path even where it fits in
-// shared memory (profiles/r05_resample.md compares the two)
-bool taps_from_global() {
-  static const bool on = [] {
-    const char* e = getenv("V100_RESAMPLE_TAPS");
-    return e != nullptr && e[0] == 'l';
-  }();
-  return on;
-}
-
 template <bool I16, bool TAPS_SMEM>
 int launch(const void* x, long long x_pitch, const int32_t* len, int L_in, const int32_t* start, const int32_t* count,
            const int32_t* off, const float* taps, int n_taps, int o, int n, int w, int JT, long long tiles, int tpc,
@@ -135,8 +121,9 @@ int launch(const void* x, long long x_pitch, const int32_t* len, int L_in, const
   if (smem > 48 * 1024) V100_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem)));
   // at least one CTA per row, which writes out_len even when the rows are empty (L_out = 0)
   const dim3 grid(static_cast<unsigned>(tiles > 0 ? (tiles + tpc - 1) / tpc : 1), static_cast<unsigned>(B));
-  V100_CUDA(launch_pdl(kern, grid, dim3(kResThreads), smem, stream, x, x_pitch, len, L_in, start, count, off, taps,
-                       n_taps, o, n, w, JT, tiles, tpc, y, y_pitch, L_out, out_len));
+  kern<<<grid, dim3(kResThreads), smem, stream>>>(x, x_pitch, len, L_in, start, count, off, taps, n_taps, o, n, w, JT,
+                                                  tiles, tpc, y, y_pitch, L_out, out_len);
+  V100_CUDA(cudaGetLastError());
   return 0;
 }
 
@@ -178,7 +165,7 @@ int resample(const void* wav, int wav_dtype, const int32_t* len, int B, int64_t 
   const int JT = G * kResR;
   const long long frames = (L_out + n - 1) / n;
   const long long tiles = (frames + JT - 1) / JT;
-  const bool tsm = n_taps <= kResMaxSmemTaps && !taps_from_global();
+  const bool tsm = n_taps <= kResMaxSmemTaps;
   // with the table in shared memory a CTA walks several tiles of its row (the table is staged once per CTA), as many
   // as keeps about 8 CTAs per SM in the grid
   int tpc = 1;

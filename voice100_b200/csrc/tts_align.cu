@@ -37,8 +37,6 @@ tts_align_kernel(const float* __restrict__ dur, long long sb, long long sl, long
                  int32_t* __restrict__ status, int32_t* __restrict__ filled_len, int32_t* __restrict__ frame_len) {
   __shared__ float2 a[kAlignMaxTokens];     // (gap, dur) of token i, then its frame range [s, e) as int2
   __shared__ int s_status, s_total, s_fill;
-  pdl_trigger();
-  pdl_wait();
   const int b = blockIdx.x;
   int n = text_len == nullptr ? L : __ldg(text_len + b);
   n = n < 0 ? 0 : (n > L ? L : n);
@@ -177,10 +175,11 @@ int tts_align(const float* durations, int64_t stride_b, int64_t stride_l, int64_
   if (L > kAlignMaxTokens)
     return fail(V100_E_UNSUPPORTED, "tts_align: L = %d tokens > %d (per-utterance token arrays in shared memory)", L,
                 kAlignMaxTokens);
-  V100_CUDA(launch_pdl(tts_align_kernel, dim3(B), dim3(kAlignThreads), 0, stream, durations, (long long)stride_b,
-                       (long long)stride_l, (long long)stride_c, log1p_input, durations_out, text,
-                       (long long)text_stride, text_len, L, rule, head, tail, aligntext, T_cap, aligntext_len, status,
-                       filled_len, frame_len));
+  tts_align_kernel<<<dim3(B), dim3(kAlignThreads), 0, stream>>>(
+      durations, (long long)stride_b, (long long)stride_l, (long long)stride_c, log1p_input, durations_out, text,
+      (long long)text_stride, text_len, L, rule, head, tail, aligntext, T_cap, aligntext_len, status, filled_len,
+      frame_len);
+  V100_CUDA(cudaGetLastError());
   return 0;
 }
 

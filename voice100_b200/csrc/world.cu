@@ -98,8 +98,6 @@ struct WorldIn {
 // ------------------------------------------------------------------------------------------------ noise table
 
 __global__ void world_noise_kernel(double* __restrict__ out, long long n) {
-  pdl_trigger();
-  pdl_wait();
   if (threadIdx.x != 0 || blockIdx.x != 0) return;
   uint32_t x = 123456789u, y = 362436069u, z = 521288629u, w = 88675123u;
   for (long long j = 0; j < n; ++j) {
@@ -151,8 +149,6 @@ world_timebase_kernel(const WorldIn in, int B, WorldWs ws, long long Yp, int32_t
   __shared__ int s_vprev;
   __shared__ int s_first[kTbThreads], s_next[kTbThreads];
   __shared__ int s_count;
-  pdl_trigger();
-  pdl_wait();
   const int b = blockIdx.x, tid = threadIdx.x;
   int Tb = in.frame_len == nullptr ? in.T : __ldg(in.frame_len + b);
   Tb = Tb < 0 ? 0 : (Tb > in.T ? in.T : Tb);
@@ -554,7 +550,6 @@ world_synth_kernel(const SynthParams P) {
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   const int b = blockIdx.y;
   const long long t0 = static_cast<long long>(blockIdx.x) * kTile;
-  pdl_trigger();
 
   for (int m = tid; m < kN; m += kSynThreads) {
     float s, c;
@@ -565,7 +560,6 @@ world_synth_kernel(const SynthParams P) {
     const double r = 0.5 - 0.5 * cos(kTwoPi * (i + 1.0) / (1.0 + kN));
     dcr[m] = static_cast<float>(r / (2.0 * (kN / 4 + 0.25)));
   }
-  pdl_wait();
   const int32_t* head = P.ws.head + 4 * b;
   const int st = head[0], y_len = head[1], first = head[2];
   float* out = P.wav + b * P.wav_pitch;
@@ -652,7 +646,8 @@ int launch_timebase(const WorldIn& in, int B, void* workspace, int32_t* wav_len,
                     cudaStream_t stream) {
   const long long Yp = ws_pitch(in.T);
   const WorldWs ws = ws_carve(workspace, B, Yp);
-  V100_CUDA(launch_pdl(world_timebase_kernel, dim3(B), dim3(kTbThreads), 0, stream, in, B, ws, Yp, wav_len, status));
+  world_timebase_kernel<<<dim3(B), dim3(kTbThreads), 0, stream>>>(in, B, ws, Yp, wav_len, status);
+  V100_CUDA(cudaGetLastError());
   return 0;
 }
 
@@ -668,7 +663,8 @@ int64_t world_workspace_bytes(int B, int64_t y_len_max) {
 int world_noise(double* out, int64_t n, cudaStream_t stream) {
   if (out == nullptr || n < 0) return fail(V100_E_INVALID, "world_noise: null output or negative length");
   if (n == 0) return 0;
-  V100_CUDA(launch_pdl(world_noise_kernel, dim3(1), dim3(32), 0, stream, out, static_cast<long long>(n)));
+  world_noise_kernel<<<dim3(1), dim3(32), 0, stream>>>(out, static_cast<long long>(n));
+  V100_CUDA(cudaGetLastError());
   return 0;
 }
 
@@ -725,8 +721,8 @@ int world_synthesize(const float* f0, int64_t f0_sb, int64_t f0_st, const float*
   p.wav_pitch = wav_pitch;
   const long long tiles = (wav_pitch + kTile - 1) / kTile;
   if (tiles > 0x7fffffffLL || B > 65535) return fail(V100_E_UNSUPPORTED, "world_synthesize: grid too large");
-  V100_CUDA(launch_pdl(world_synth_kernel, dim3(static_cast<unsigned>(tiles), B), dim3(kSynThreads), kSynSmem, stream,
-                       p));
+  world_synth_kernel<<<dim3(static_cast<unsigned>(tiles), B), dim3(kSynThreads), kSynSmem, stream>>>(p);
+  V100_CUDA(cudaGetLastError());
   return 0;
 }
 

@@ -179,27 +179,6 @@ def dwconv(x: Ncw, w: torch.Tensor, scale, shift, k: int, stride: int, act: int,
     return y
 
 
-def dw_pack_pairs(w: torch.Tensor) -> torch.Tensor:
-    """Depthwise filter [C, k] (16-bit) -> the packed pair table [C, 128] int32 that v100_expand_dw reads."""
-    _cuda(w)
-    dt(w)
-    C, k = w.shape
-    out = torch.empty((C, 128), device=w.device, dtype=torch.int32)
-    _call(w, "v100_dw_pack_pairs", w.data_ptr(), out.data_ptr(), C, k)
-    return out
-
-
-def expand_dw(x: Ncw, W1: torch.Tensor, s1, b1, dw_pairs: torch.Tensor, s2, b2, k: int) -> Ncw:
-    """Fused pointwise expand (+BN+ReLU6) and depthwise k (+BN+ReLU6), stride 1: x [B, C_in, T] -> y [B, H, T]."""
-    H, C_in = W1.shape
-    assert C_in == x.C and W1.dtype == x.data.dtype and dw_pairs.shape == (H, 128)
-    _same_device(x, W1, s1, b1, dw_pairs, s2, b2)
-    y = empty_ncw(x.B, H, x.T, x.data.device, x.data.dtype)
-    _call(x, "v100_expand_dw", x.data.data_ptr(), x.pitch, W1.data_ptr(), _ptr(s1), b1.data_ptr(), dw_pairs.data_ptr(),
-          _ptr(s2), b2.data_ptr(), y.data.data_ptr(), y.pitch, x.B, C_in, H, x.T, k, dt(x.data))
-    return y
-
-
 def convtranspose_k5s2(x: Ncw, Wp: torch.Tensor, bias: torch.Tensor) -> Ncw:
     C_out = Wp.shape[0]
     assert Wp.shape[1] == 5 * x.C and Wp.dtype == x.data.dtype
