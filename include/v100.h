@@ -474,6 +474,57 @@ int v100_resample(const void* wav, int wav_dtype, const int32_t* len, int B, int
                   const int32_t* start, const int32_t* count, const int32_t* off, const float* taps, int n_taps,
                   int o, int n, int w, float* out, int64_t out_pitch, int64_t L_out, int32_t* out_len, void* stream);
 
+/* ------------------------------------------------------------------------------------------------
+ * ASR evaluation: CTC loss and token edit distance
+ * ------------------------------------------------------------------------------------------------ */
+
+/* per-utterance status codes of v100_ctc_loss */
+#define V100_CTC_OK         0
+#define V100_CTC_BAD_LABEL  1   /* a target label outside [0, V) (torch's CPU kernel reads out of bounds)       */
+#define V100_CTC_BAD_LENGTH 2   /* input length outside [0, T], target length outside [0, L_max], or a target
+                                   running past the end of the target buffer (torch raises RuntimeError)        */
+#define V100_CTC_MAX_TARGET 4096   /* L_max limit of v100_ctc_loss (V100_E_UNSUPPORTED above)                   */
+#define V100_EDIT_MAX_LEN   16384  /* width limit of v100_edit_distance on either side (V100_E_UNSUPPORTED above) */
+
+/*
+ * CTC loss per utterance: torch.nn.functional.ctc_loss(..., reduction="none"), the criterion the reference evaluates
+ * with (self.loss_fn = nn.CTCLoss(zero_infinity=True), voice100/models/asr.py:105-106, _calc_batch_loss at
+ * asr.py:133-152).  The forward algorithm over the 2l+1 blank-expanded states runs in log space in float64 (and so
+ * does the log_softmax when normalize != 0); the result is rounded to fp32 once.  Semantics as torch 2.11 on the CPU:
+ * the skip into an odd state s >= 3 is allowed iff target[(s-1)/2] != target[(s-3)/2]; a label equal to `blank` is an
+ * ordinary label; too few frames for the target (input length 0 with a non-empty target included) gives +inf;
+ * input length 0 with target length 0 gives 0; target length 0 gives -sum_t log p_t(blank).
+ *   x          fp32 scores, element (t, b, v) at x[t*stride_t + b*stride_b + v] (unit stride along V): log-probabilities,
+ *              or raw logits with normalize != 0 (the kernel applies log_softmax over V).  The v1 logits [B][T][V]
+ *              are (V, T*V); time-major logits [T][Bp][V] are (Bp*V, V)
+ *   input_len  int32 [B] on the device;  target_len int32 [B] on the device
+ *   targets    int64; utterance b's labels are targets[off_b .. off_b + target_len[b]) with off_b = target_off[b] when
+ *              target_off (int64 [B]) is given (torch's concatenated 1-D form), else b * target_stride (the padded
+ *              [B][S] form); targets_numel = elements of the buffer;  L_max = the largest target length allowed
+ *              (<= V100_CTC_MAX_TARGET; it sizes shared memory)
+ *   zero_infinity  != 0: +inf becomes 0
+ *   loss       fp32 [B];  status  optional int32 [B]: V100_CTC_*; a bad utterance's loss is NaN
+ * V <= 8192.  One CTA per utterance; no host synchronisation, no atomics, CUDA-graph capturable; a result does not
+ * depend on the rest of the batch and is bit-identical from run to run.
+ */
+int v100_ctc_loss(const float* x, int64_t stride_t, int64_t stride_b, int T, int B, int V, const int32_t* input_len,
+                  const int64_t* targets, int64_t target_stride, const int64_t* target_off, int64_t targets_numel,
+                  const int32_t* target_len, int L_max, int blank, int normalize, int zero_infinity, float* loss,
+                  int32_t* status, void* stream);
+
+/*
+ * Levenshtein distance with unit costs between int64 id sequences (token or, with words mapped to ids on the host,
+ * word errors of the reference's greedy transcripts, voice100/models/asr.py:133-152).  Any int64 value is a valid id.
+ *   hyp  [B][hyp_stride] with hyp_len int32 [B] (NULL = hyp_width);  ref [B][ref_stride] with ref_len (NULL = ref_width);
+ *        lengths are clamped to [0, width] on the device, as v100_ctc_collapse does
+ *   dist int32 [B]
+ * Widths <= V100_EDIT_MAX_LEN.  One CTA per pair, anti-diagonal DP in shared memory: exact, deterministic, no host
+ * synchronisation, CUDA-graph capturable.
+ */
+int v100_edit_distance(const int64_t* hyp, int64_t hyp_stride, const int32_t* hyp_len, int hyp_width,
+                       const int64_t* ref, int64_t ref_stride, const int32_t* ref_len, int ref_width, int B,
+                       int32_t* dist, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -46,6 +46,8 @@ SIGNATURES = {
     "v100_resample": [_p, _i, _p, _i, _l, _l, _p, _p, _p, _p, _i, _i, _i, _i, _p, _l, _l, _p, _p],
     "v100_world_analysis_workspace_bytes": [_i, _l],   # returns int64 (restype set in lib())
     "v100_world_analyze": [_p, _i, _l, _p, _i, _l, _p, _p, _l, _p, _i, _p, _p, _p, _p, _p, _p],
+    "v100_ctc_loss": [_p, _l, _l, _i, _i, _i, _p, _p, _l, _p, _l, _p, _i, _i, _i, _i, _p, _p, _p],
+    "v100_edit_distance": [_p, _l, _p, _i, _p, _l, _p, _i, _i, _p, _p],
 }
 
 ABI_VERSION = 9

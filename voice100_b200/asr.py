@@ -129,6 +129,31 @@ class AsrPipeline:
         return K.ctc_collapse(tokens, out_len, blank)
 
     @torch.no_grad()
+    def evaluate(self, waveform: torch.Tensor, lengths: torch.Tensor, text: torch.Tensor, text_len,
+                 sample_rate: Optional[int] = None, blank: int = 0):
+        """Score a batch against its transcripts, as the reference's validation / test steps do (forward ->
+        log_softmax -> nn.CTCLoss(zero_infinity=True), voice100/models/asr.py:105-106,133-152), plus the token errors of
+        the greedy transcripts.  text int64 [B, S] padded, text_len [B] (device tensor or host sequence).
+        -> (loss fp32 [B] per utterance with zero_infinity, errors int32 [B] = edit distance between the collapsed
+        greedy ids and text, ids, counts), where (ids, counts) are exactly what `transcribe_ids` returns.  The batch
+        loss the reference logs is `(loss / text_len.clamp_min(1)).mean()`.  v1: log-mel -> encoder -> CTC tail with
+        logits -> ctc_loss on those logits in place (log_softmax inside) -> collapse -> edit distance, 33 launches
+        and no host synchronisation (capturable when text_len is a device tensor)."""
+        feats, audio_len = self.transform.logmel_batch(waveform, lengths, ncw_dtype=self.model.storage_dtype,
+                                                       orig_freq=self._rate(sample_rate))
+        m = self.model
+        logits, tokens, out_len = K.ctc_finalize(m.decoder.run(m.encoder.run(feats)), True, audio_len)
+        return self._score(logits.transpose(0, 1), tokens, out_len, text, text_len, blank)
+
+    @staticmethod
+    def _score(logits_tbv, tokens, out_len, text, text_len, blank):
+        """logits [T', B, V] (a view), greedy tokens int64 [B, T'], valid lengths [B] -> evaluate's four results."""
+        loss = K.ctc_loss_batch(logits_tbv, text, out_len, text_len, blank=blank, zero_infinity=True,
+                                normalize=True)[0]
+        ids, counts = K.ctc_collapse(tokens, out_len, blank)
+        return loss, K.edit_distance(ids, counts, text, text_len), ids, counts
+
+    @torch.no_grad()
     def _capture(self, batch: int, samples: int, dev, wav_dtype=torch.float32, sample_rate=None):
         """-> (graph, static waveform, static lengths, static tokens, static out_len) for one fixed shape.  With a
         `sample_rate` the resampled buffer inside the graph is [batch, ceil(n samples / o)]."""

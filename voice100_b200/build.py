@@ -13,7 +13,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libv100.so")
 SOURCES = ["api.cu", "conv_gemm.cu", "dwconv.cu", "logmel.cu", "misc.cu", "seq.cu", "lstm.cu", "tts_align.cu",
-           "world.cu", "resample.cu", "world_analysis.cu"]
+           "world.cu", "resample.cu", "world_analysis.cu", "ctc_eval.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "--compiler-options", "-fPIC", "-shared"]
 

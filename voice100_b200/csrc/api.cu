@@ -269,4 +269,19 @@ int v100_resample(const void* wav, int wav_dtype, const int32_t* len, int B, int
                   L_out, out_len, STREAM(stream));
 }
 
+int v100_ctc_loss(const float* x, int64_t stride_t, int64_t stride_b, int T, int B, int V, const int32_t* input_len,
+                  const int64_t* targets, int64_t target_stride, const int64_t* target_off, int64_t targets_numel,
+                  const int32_t* target_len, int L_max, int blank, int normalize, int zero_infinity, float* loss,
+                  int32_t* status, void* stream) {
+  return ctc_loss(x, stride_t, stride_b, T, B, V, input_len, targets, target_stride, target_off, targets_numel,
+                  target_len, L_max, blank, normalize, zero_infinity, loss, status, STREAM(stream));
+}
+
+int v100_edit_distance(const int64_t* hyp, int64_t hyp_stride, const int32_t* hyp_len, int hyp_width,
+                       const int64_t* ref, int64_t ref_stride, const int32_t* ref_len, int ref_width, int B,
+                       int32_t* dist, void* stream) {
+  return edit_distance(hyp, hyp_stride, hyp_len, hyp_width, ref, ref_stride, ref_len, ref_width, B, dist,
+                       STREAM(stream));
+}
+
 }  // extern "C"

@@ -108,4 +108,13 @@ int resample(const void* wav, int wav_dtype, const int32_t* len, int B, int64_t 
              const int32_t* start, const int32_t* count, const int32_t* off, const float* taps, int n_taps, int o,
              int n, int w, float* out, int64_t out_pitch, int64_t L_out, int32_t* out_len, cudaStream_t stream);
 
+// ASR evaluation (ctc_eval.cu)
+int ctc_loss(const float* x, int64_t stride_t, int64_t stride_b, int T, int B, int V, const int32_t* input_len,
+             const int64_t* targets, int64_t target_stride, const int64_t* target_off, int64_t targets_numel,
+             const int32_t* target_len, int L_max, int blank, int normalize, int zero_infinity, float* loss,
+             int32_t* status, cudaStream_t stream);
+int edit_distance(const int64_t* hyp, int64_t hyp_stride, const int32_t* hyp_len, int hyp_width, const int64_t* ref,
+                  int64_t ref_stride, const int32_t* ref_len, int ref_width, int B, int32_t* dist,
+                  cudaStream_t stream);
+
 }  // namespace v100

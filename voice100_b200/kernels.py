@@ -701,3 +701,146 @@ def resample(wav: torch.Tensor, lengths: torch.Tensor, table, L_out: int):
           table.start.data_ptr(), table.count.data_ptr(), table.off.data_ptr(), _ptr(table.taps), table.taps.numel(),
           table.o, table.n, table.width, out.data_ptr(), L_out, L_out, out_len.data_ptr())
     return out, out_len
+
+
+# ---------------------------------------------------------------------------------------------- ASR evaluation
+
+CTC_OK, CTC_BAD_LABEL, CTC_BAD_LENGTH = 0, 1, 2       # V100_CTC_*
+CTC_MAX_TARGET = 4096                                 # V100_CTC_MAX_TARGET
+EDIT_MAX_LEN = 16384                                  # V100_EDIT_MAX_LEN
+
+
+def _host_lengths(x):
+    """Host-resident lengths (list, tuple, CPU tensor) as a Python list; None for a device tensor."""
+    if isinstance(x, torch.Tensor) and x.is_cuda:
+        return None
+    return [int(v) for v in (x.tolist() if isinstance(x, torch.Tensor) else x)]
+
+
+def _lengths_i32(x, device, what: str, B: int):
+    """Lengths as a device int32 [B] tensor.  Device values are not read back: they are clamped into the int32 range,
+    so that an out-of-range value stays out of range for the kernel's own check."""
+    vals = _host_lengths(x)
+    if vals is None:
+        if x.device != device:
+            raise _lib.V100Error(f"{what} lives on {x.device}, the other operands on {device}")
+        if x.shape != (B,):
+            raise _lib.V100Error(f"{what} must have shape [{B}], got {tuple(x.shape)}")
+        return (x if x.dtype == torch.int32 else x.clamp(-1, 2 ** 31 - 1).to(torch.int32)).contiguous()
+    if len(vals) != B:
+        raise RuntimeError(f"{what} must be of size batch_size = {B}, got {len(vals)}")
+    return torch.tensor([min(max(v, -1), 2 ** 31 - 1) for v in vals], dtype=torch.int32).to(device)
+
+
+def ctc_loss_batch(log_probs: torch.Tensor, targets: torch.Tensor, input_lengths, target_lengths, blank: int = 0,
+                   zero_infinity: bool = False, normalize: bool = False):
+    """One v100_ctc_loss call -> (loss fp32 [N], status int32 [N] = CTC_*, target lengths int32 [N] on the device).
+    log_probs fp32 [T, N, C] on the device with unit stride along C (any other strides are read in place); targets
+    int64 [N, S] (padded) or 1-D (concatenated); lengths as torch accepts them.  Host-resident lengths are checked
+    before anything else, raising RuntimeError where torch does; device-resident ones are checked by the kernel (NaN
+    and CTC_BAD_LENGTH)."""
+    if not isinstance(log_probs, torch.Tensor) or log_probs.dtype != torch.float32 or log_probs.dim() != 3:
+        raise _lib.V100Error("ctc_loss: log_probs must be an fp32 [T, N, C] tensor")
+    T, B, V = log_probs.shape
+    if B == 0 or T == 0:
+        raise _lib.V100Error("ctc_loss: empty batch")
+    if not 0 <= blank < V:
+        raise RuntimeError("blank must be in label range")
+    if not isinstance(targets, torch.Tensor) or targets.dim() not in (1, 2) or targets.is_floating_point():
+        raise RuntimeError("ctc_loss: targets must be an integer tensor [N, S] or 1-D")
+    il_host, tl_host = _host_lengths(input_lengths), _host_lengths(target_lengths)
+    for what, vals in (("input_lengths", il_host), ("target_lengths", tl_host)):
+        if vals is not None and len(vals) != B:
+            raise RuntimeError(f"{what} must be of size batch_size = {B}, got {len(vals)}")
+        if vals is not None and min(vals) < 0:
+            raise RuntimeError(f"Expected {what} to have value at least 0, but got value {min(vals)}")
+    if il_host is not None and max(il_host) > T:
+        raise RuntimeError(f"Expected input_lengths to have value at most {T}, but got value {max(il_host)}")
+    if targets.dim() == 2:
+        if targets.shape[0] != B:
+            raise RuntimeError(f"ctc_loss: targets has {targets.shape[0]} rows for a batch of {B}")
+        if tl_host is not None and max(tl_host) > targets.shape[1]:
+            raise RuntimeError(f"Expected tensor to have size at least {max(tl_host)} at dimension 1, but got size "
+                               f"{targets.shape[1]} for argument #2 'targets'")
+    elif tl_host is not None and sum(tl_host) > targets.numel():
+        raise RuntimeError(f"Expected tensor to have size at least {sum(tl_host)} at dimension 0, but got size "
+                           f"{targets.numel()} for argument #2 'targets'")
+    if not log_probs.is_cuda:
+        raise _lib.V100Error("ctc_loss: voice100_b200 kernels need CUDA tensors (there is no CPU path)")
+    if log_probs.stride(2) != 1 and V > 1:
+        raise _lib.V100Error("ctc_loss: log_probs needs unit stride along C")
+    dev = log_probs.device
+    targets = targets.to(device=dev, dtype=torch.int64)
+    il = _lengths_i32(input_lengths, dev, "input_lengths", B)
+    tl = _lengths_i32(target_lengths, dev, "target_lengths", B)
+    off = None
+    if targets.dim() == 2:
+        if targets.shape[1] > 0 and targets.stride(1) != 1:
+            targets = targets.contiguous()
+        stride, L_max = targets.stride(0), targets.shape[1]
+        numel = (B - 1) * stride + targets.shape[1] if targets.shape[1] else 0
+        if tl_host is not None:
+            L_max = max(tl_host)                          # known lengths: a wide padded buffer is not a limit
+    else:
+        targets = targets.contiguous()
+        stride, numel = 0, targets.numel()
+        if tl_host is not None:
+            L_max = max(tl_host)
+            off = torch.tensor([sum(tl_host[:b]) for b in range(B)], dtype=torch.int64).to(dev)
+        else:
+            L_max = min(numel, CTC_MAX_TARGET)
+            t64 = tl.to(torch.int64)
+            off = (torch.cumsum(t64, 0) - t64).contiguous()
+    loss = torch.empty((B,), device=dev, dtype=torch.float32)
+    status = torch.empty((B,), device=dev, dtype=torch.int32)
+    _call(log_probs, "v100_ctc_loss", log_probs.data_ptr(), log_probs.stride(0), log_probs.stride(1), T, B, V,
+          il.data_ptr(), targets.data_ptr() if targets.numel() else None, stride, _ptr(off), numel, tl.data_ptr(),
+          int(L_max), int(blank), 1 if normalize else 0, 1 if zero_infinity else 0, loss.data_ptr(),
+          status.data_ptr())
+    return loss, status, tl
+
+
+def ctc_loss(log_probs: torch.Tensor, targets: torch.Tensor, input_lengths, target_lengths, blank: int = 0,
+             reduction: str = "mean", zero_infinity: bool = False, normalize: bool = False) -> torch.Tensor:
+    """torch.nn.functional.ctc_loss on the device (v100_ctc_loss): the forward algorithm in float64, the result in fp32.
+    Same signature, layout ([T, N, C] log-probabilities, any strides with unit stride along C) and results as torch's
+    CPU kernel; `normalize=True` takes raw logits and applies log_softmax in the kernel (float64), so the logits of the
+    ASR heads are read in place.  reduction "none" -> fp32 [N]; "mean" -> (loss / target_lengths.clamp_min(1)).mean();
+    "sum" -> loss.sum() (torch's own expressions on the per-utterance vector).  A target label outside [0, C) or a
+    device-resident length out of range gives NaN for that utterance; host-resident lengths out of range raise
+    RuntimeError before launch, as torch does.  No backward: this is for evaluation."""
+    if reduction not in ("none", "mean", "sum"):
+        raise ValueError(f"{reduction} is not a valid value for reduction")
+    loss, _, tl = ctc_loss_batch(log_probs, targets, input_lengths, target_lengths, blank, zero_infinity, normalize)
+    if reduction == "none":
+        return loss
+    if reduction == "sum":
+        return loss.sum()
+    return (loss / tl.to(loss.dtype).clamp_min(1)).mean()
+
+
+def edit_distance(hyp: torch.Tensor, hyp_len, ref: torch.Tensor, ref_len) -> torch.Tensor:
+    """Levenshtein distance with unit costs between int64 id sequences on the device (v100_edit_distance).
+    hyp int64 [B, Lh], ref int64 [B, Lr] (row strides free, unit stride along the row), hyp_len / ref_len [B] (device
+    tensors, host sequences or None = the full width; clamped to [0, width] as ctc_collapse does) -> int32 [B].
+    Any int64 is a valid id, so word errors are this function on word ids mapped on the host."""
+    for name, t in (("hyp", hyp), ("ref", ref)):
+        if not isinstance(t, torch.Tensor) or not t.is_cuda:
+            raise _lib.V100Error(f"edit_distance: {name} must be a CUDA tensor (there is no CPU path)")
+        if t.dtype != torch.int64 or t.dim() != 2:
+            raise _lib.V100Error(f"edit_distance: {name} must be int64 [B, L], got {t.dtype} {tuple(t.shape)}")
+    _same_device(hyp, ref)
+    B = hyp.shape[0]
+    if ref.shape[0] != B or B == 0:
+        raise _lib.V100Error(f"edit_distance: batch sizes {B} and {ref.shape[0]} differ or are 0")
+    if hyp.shape[1] > EDIT_MAX_LEN or ref.shape[1] > EDIT_MAX_LEN:
+        raise _lib.V100Error(f"edit_distance: widths {hyp.shape[1]} / {ref.shape[1]} exceed {EDIT_MAX_LEN}")
+    hyp = hyp if hyp.shape[1] == 0 or hyp.stride(1) == 1 else hyp.contiguous()
+    ref = ref if ref.shape[1] == 0 or ref.stride(1) == 1 else ref.contiguous()
+    dev = hyp.device
+    hl = None if hyp_len is None else _lengths_i32(hyp_len, dev, "hyp_len", B)
+    rl = None if ref_len is None else _lengths_i32(ref_len, dev, "ref_len", B)
+    dist = torch.empty((B,), device=dev, dtype=torch.int32)
+    _call(hyp, "v100_edit_distance", hyp.data_ptr() if hyp.numel() else None, hyp.stride(0), _ptr(hl), hyp.shape[1],
+          ref.data_ptr() if ref.numel() else None, ref.stride(0), _ptr(rl), ref.shape[1], B, dist.data_ptr())
+    return dist

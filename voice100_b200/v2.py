@@ -254,6 +254,20 @@ class AsrV2Pipeline(AsrPipeline):
         tokens, x_len = self.model.greedy(feats, audio_len)
         return tokens.t().contiguous(), x_len
 
+    @torch.no_grad()
+    def evaluate(self, waveform: torch.Tensor, lengths: torch.Tensor, text: torch.Tensor, text_len,
+                 sample_rate: Optional[int] = None, blank: int = 0):
+        """AsrPipeline.evaluate for AudioToAlignText: the CTC tail writes the head's logits time-major ([T, Bp, V]) and
+        the loss kernel reads the first B columns of each step in place.  Same results as AsrPipeline.evaluate."""
+        feats, audio_len = self.transform.logmel_batch(waveform, lengths, ncw_dtype=self.model.storage_dtype,
+                                                       orig_freq=self._rate(sample_rate))
+        x_len = self.model.output_length(audio_len)
+        y, tm = self.model._run(feats, x_len)
+        logits, tokens = K.ctc_finalize(y, want_logits=True)        # [1, T*Bp, V], [1, T*Bp]
+        logits = logits.view(tm.T, tm.Bp, y.C)[:, :tm.B]
+        tokens = tokens.view(tm.T, tm.Bp)[:, :tm.B].t().contiguous()
+        return self._score(logits, tokens, x_len, text, text_len, blank)
+
 
 class TextToAlignText(StorageDtypeMixin, nn.Module):
     """Duration model of align_*.yaml (_align_v2.py:17-82)."""
